@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: the regularised-DAE train step (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--precision P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--precision P] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the train path over one batch of 4096 synthetic cubes per GPU:
@@ -531,6 +531,30 @@ def oracle_loss_check(eng, csr, batch_ids, prob, alias, indptr, indices, W, log)
                     "M-hat rows from the oracle's own counts", "seconds": time.time() - t0}
 
 
+DUMP_SAMPLE = 1 << 20      # entries kept of a larger weight tensor: the three C x 512 kernels are 128 MB in full
+
+
+def dump_outputs(out_dir, loss, weights, log):
+    """What a caller of the train step receives from the last timed step: loss3 = [bce, kl, total] (float64) and every
+    weight tensor after its Adam update (float32, Keras names with '/' -> '.'), one <name>.npy each.  A tensor of more
+    than DUMP_SAMPLE entries is written as `<name>.sampled.npy`: the same DUMP_SAMPLE flat positions in every run.
+    The inputs are seeded, but the bias gradients and the first layer's backward sum with float atomics, and Adam's
+    m / sqrt(v) turns those rounding differences of near-zero gradients into +-lr weight steps: two runs of one build
+    agree on the first step's loss and drift apart from there (on a B200 after 25 steps: loss 1e-3 relative, weights up
+    to 1.1e-2), so builds are compared with a tolerance, not bit for bit."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.cpu().numpy().astype(np.float64))
+    total = 0
+    for key, w in weights.items():
+        name = key.replace("/", ".")
+        if w.size > DUMP_SAMPLE:
+            pick = np.sort(np.random.default_rng(0).choice(w.size, DUMP_SAMPLE, replace=False))
+            w, name = w.ravel()[pick], name + ".sampled"
+        np.save(os.path.join(out_dir, name + ".npy"), w.astype(np.float32))
+        total += w.nbytes
+    log(f"outputs of the last timed step: {len(weights) + 1} arrays, {total / 2**20:.1f} MB -> {out_dir}")
+
+
 def run_native(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -613,6 +637,8 @@ def run_native(args, rank, world, local_rank):
     ev1.record()
     barrier()
     clocks.mark_end()
+    # the last timed step's results, held before the instrumented pass below trains the model further
+    outputs = (loss.clone(), model.store.params.clone()) if args.dump_outputs and rank == 0 else None
     ms = torch.tensor([ev0.elapsed_time(ev1)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -683,6 +709,8 @@ def run_native(args, rank, world, local_rank):
         if world > 1:
             dist.destroy_process_group()
         return
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs[0], model.store.to_dict(outputs[1]), log)
     # ---- roofline of the dominant kernel: the eight 512<->C GEMM passes per step (seven with the gather first layer) ----
     peaks = load_peaks()
     n_big, ms_big = ktimes.get("big_gemm", (0, 0.0))
@@ -779,7 +807,14 @@ def main():
     ap.add_argument("--no-loss-check", action="store_true", help="N = 1: skip the float64 oracle comparison of the step-1 loss")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the graph-build and ml_recommend side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and the updated weights of the last timed step to DIR/<name>.npy (inputs are "
+                         "seeded: two builds run with the same arguments can be compared array by array)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the outputs of the native train step (--impl native)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
