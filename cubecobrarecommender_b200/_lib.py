@@ -91,6 +91,7 @@ SIGNATURES = {
     "cc_softmax_kl_set_variant": (I, [I]),
     "cc_softmax_kl_fwd_bwd_metrics": (I, [P, I64, P, I64, P, I32, I32, I32, D, P, I64, P, I, P, P, I64, P, P, P, P]),
     "cc_kl_target_argmax": (I, [P, I64, I32, I32, P, P]),
+    "cc_softmax_kl_loss": (I, [P, I64, P, I64, P, I32, I32, I32, P, P, P, P, I, P]),
     "cc_binary_accuracy_rows": (I, [P, I64, P, I64, I32, I32, P, P]),
     "cc_convert_f32_bf16": (I, [P, I64, P, I64, I32, I32, P]),
     "cc_loss_finalize": (I, [P, I32, D, P, I32, D, D, P, P]),

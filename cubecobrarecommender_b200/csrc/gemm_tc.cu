@@ -24,6 +24,7 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <stdlib.h>
+#include <string.h>
 
 #include <atomic>
 #include <mutex>
@@ -55,7 +56,10 @@ template <int BN, int CTAS> struct Cfg {
 // EPI_BCE16: the fused sigmoid-BCE epilogue writing dlogits as bf16 (they feed the bf16 dW / dX GEMMs of the "bf16" mode)
 // EPI_BCE_ACC / EPI_BCE16_ACC: the same two with the Keras binary_accuracy count (four more instructions per element,
 // compiled in only when the caller asks for metrics)
-enum Epilogue : int { EPI_STORE = 0, EPI_BCE = 1, EPI_COUNT = 2, EPI_BCE16 = 3, EPI_BCE_ACC = 4, EPI_BCE16_ACC = 5 };
+// EPI_BCE_LOSS / EPI_BCE_LOSS_ACC: loss (and accuracy) partials only, for evaluation: no dlogits, no C tensor map, no
+// bias-gradient sums
+enum Epilogue : int { EPI_STORE = 0, EPI_BCE = 1, EPI_COUNT = 2, EPI_BCE16 = 3, EPI_BCE_ACC = 4, EPI_BCE16_ACC = 5,
+                      EPI_BCE_LOSS = 6, EPI_BCE_LOSS_ACC = 7 };
 // operand kinds: fp32 storage / kind::tf32, bf16 storage / kind::f16, uint8 storage / kind::i8 (int32 accumulators:
 // the co-occurrence contraction X^T X over 0/1 bytes is exact)
 enum Kind : int { KIND_TF32 = 0, KIND_BF16 = 1, KIND_U8 = 2 };
@@ -335,9 +339,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
                const __grid_constant__ CUtensorMap map_c, const Params p) {
   using C = Cfg<BN, CTAS>;
   constexpr bool BF16 = KIND == KIND_BF16;
-  constexpr bool IS_BCE = EPI == EPI_BCE || EPI == EPI_BCE16 || EPI == EPI_BCE_ACC || EPI == EPI_BCE16_ACC;
+  constexpr bool LOSS_ONLY = EPI == EPI_BCE_LOSS || EPI == EPI_BCE_LOSS_ACC;      // nothing is stored but the partials
+  constexpr bool IS_BCE = EPI == EPI_BCE || EPI == EPI_BCE16 || EPI == EPI_BCE_ACC || EPI == EPI_BCE16_ACC || LOSS_ONLY;
   constexpr bool OUT16 = EPI == EPI_BCE16 || EPI == EPI_BCE16_ACC;   // output elements are bf16 (32 x 32 block = 64-byte rows)
-  constexpr bool WANT_ACC = EPI == EPI_BCE_ACC || EPI == EPI_BCE16_ACC;
+  constexpr bool WANT_ACC = EPI == EPI_BCE_ACC || EPI == EPI_BCE16_ACC || EPI == EPI_BCE_LOSS_ACC;
   constexpr int BN_LOAD = BN / CTAS;             // rows of the B tile this CTA stages
   constexpr int STAGES = C::STAGES;
   constexpr int STAGE_BYTES = C::STAGE_BYTES;
@@ -375,7 +380,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   if (warp == 0 && lane == 0) {
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a) : "memory");
     asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_c) : "memory");
+    if constexpr (!LOSS_ONLY) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_c) : "memory");
   }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
@@ -655,18 +660,18 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
             }
             const float e = exp2f_approx(-1.4426950408889634f * fabsf(z));
             const float s1 = 1.f + e;
-            const float r = rcp_approx(s1);
+            const float r = LOSS_ONLY ? 0.f : rcp_approx(s1);
             const float lin = fmaf(-z, y, fmaxf(z, 0.f));
             row_loss += live ? lin : 0.f;
             prod *= live ? s1 : 1.f;
-            g = ((z >= 0.f ? r : e * r) - y) * inv_row;
+            if constexpr (!LOSS_ONLY) g = ((z >= 0.f ? r : e * r) - y) * inv_row;
           };
           if (col0 + 32 <= p.n) {                       // warp-uniform: only the last column tile is ragged
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
               float g;
               bce_elem(j, true, g);
-              out[j] = p.round_tf32 ? rn_tf32_bits(g) : g;
+              if constexpr (!LOSS_ONLY) out[j] = p.round_tf32 ? rn_tf32_bits(g) : g;
             }
           } else {
 #pragma unroll
@@ -674,11 +679,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
               float g;
               const bool live = (col0 + j < p.n);
               bce_elem(j, live, g);
-              g = live ? g : 0.f;
-              out[j] = p.round_tf32 ? rn_tf32_bits(g) : g;
+              if constexpr (!LOSS_ONLY) {
+                g = live ? g : 0.f;
+                out[j] = p.round_tf32 ? rn_tf32_bits(g) : g;
+              }
             }
           }
           row_loss = fmaf(0.6931471805599453f, lg2_approx(prod), row_loss);
+          if constexpr (LOSS_ONLY) continue;
         } else {
           // branch-free inner loops: bias is 0 when absent, ReLU is a max with -inf when off
           const float floor_v = p.relu ? 0.f : -INFINITY;
@@ -1023,7 +1031,8 @@ static int launch_bn(const Problem& pr, Params p, cudaStream_t st) {
   else                rc = make_map(&map_b, pr.b, elem, mt, pr.k, pr.n, pr.ldb, bk, TF32);
   if (rc != CC_OK) return rc;
   // C: fp32 (int32 counts) [M][n_store] boxes of 32 rows x 32 columns (TMA clips rows >= M and columns >= n_store)
-  if (EPI == EPI_BCE16 || EPI == EPI_BCE16_ACC) rc = make_map(&map_c, pr.c, 2, MAP_BF16, pr.m, p.n_store, pr.ldc, 32, false, 32);
+  if constexpr (EPI == EPI_BCE_LOSS || EPI == EPI_BCE_LOSS_ACC) { memset(&map_c, 0, sizeof(map_c)); rc = CC_OK; }   // never read
+  else if (EPI == EPI_BCE16 || EPI == EPI_BCE16_ACC) rc = make_map(&map_c, pr.c, 2, MAP_BF16, pr.m, p.n_store, pr.ldc, 32, false, 32);
   else rc = make_map(&map_c, pr.c, 4, EPI == EPI_COUNT ? MAP_S32 : MAP_F32, pr.m, p.n_store, pr.ldc, 32, false);
   if (rc != CC_OK) return rc;
   p.a_mn_major = pr.transa ? 1 : 0;
@@ -1531,6 +1540,8 @@ int cc_gemm_tc(int precision, int transa, int transb, int m, int n, int k, const
 // Fused decoder output layer + sigmoid-BCE:  z = A[M,K] W[K,N] + bias;  loss partials and
 // dlogits = (sigmoid(z) - y)/count written to dz[M][lddz] (columns [N, lddz) zeroed).
 // loss_partial: float64 [cc_gemm_bce_partial_count(m, lddz)]  (sum it with cc_loss_finalize).
+// dz == NULL: loss only (evaluation) -- the partials are the same, nothing else is written; lddz still sizes the
+// partial array, dbias must be NULL and dz_bf16 0.
 int cc_gemm_bce_tc(int precision, int m, int n, int k, const void* a, int64_t lda, const void* w, int64_t ldw,
                    const float* bias, const uint32_t* ybits, int64_t ywords, double count, void* dz, int64_t lddz,
                    double* loss_partial, float* dbias, int round_tf32, int dz_bf16, void* stream) {
@@ -1544,7 +1555,8 @@ int cc_gemm_bce_tc_ex(int precision, int m, int n, int k, const void* a, int64_t
                       const float* bias, const uint32_t* ybits, int64_t ywords, double count, void* dz, int64_t lddz,
                       double* loss_partial, float* dbias, int round_tf32, int dz_bf16, double* acc_partial, void* stream) {
   CC_NVTX("cc_gemm_bce_tc");
-  CC_REQUIRE(a && w && bias && ybits && dz && loss_partial, "cc_gemm_bce_tc: null pointer");
+  CC_REQUIRE(a && w && bias && ybits && loss_partial, "cc_gemm_bce_tc: null pointer");
+  CC_REQUIRE(dz || (!dbias && !dz_bf16), "cc_gemm_bce_tc: loss only (dz == NULL) takes no dbias and no bf16 dlogits");
   CC_REQUIRE(precision == 1 || precision == 2, "cc_gemm_bce_tc: precision must be 1 (tf32) or 2 (bf16)");
   CC_REQUIRE(m > 0 && n > 0 && k > 0 && count > 0, "cc_gemm_bce_tc: bad sizes");
   CC_REQUIRE(lddz % 32 == 0 && lddz >= n && ywords * 32 >= lddz,
@@ -1558,6 +1570,14 @@ int cc_gemm_bce_tc_ex(int precision, int m, int n, int k, const void* a, int64_t
   if (dbias) CC_CHECK_CUDA(cudaMemsetAsync(dbias, 0, size_t(n) * sizeof(float), as_stream(stream)));
   tc::Problem pr{0, 0, m, n, k, a, lda, w, ldw, static_cast<float*>(dz), lddz, precision == 2 ? tc::KIND_BF16 : tc::KIND_TF32};
   const int ctas = tc::g_pair_mode == 0 ? 1 : 2;
+  if (!dz) {
+    if (acc_partial) {
+      if (precision == 2) return tc::launch<tc::KIND_BF16, tc::EPI_BCE_LOSS_ACC>(pr, p, 256, ctas, as_stream(stream));
+      return tc::launch<tc::KIND_TF32, tc::EPI_BCE_LOSS_ACC>(pr, p, 256, ctas, as_stream(stream));
+    }
+    if (precision == 2) return tc::launch<tc::KIND_BF16, tc::EPI_BCE_LOSS>(pr, p, 256, ctas, as_stream(stream));
+    return tc::launch<tc::KIND_TF32, tc::EPI_BCE_LOSS>(pr, p, 256, ctas, as_stream(stream));
+  }
   if (dz_bf16) {
     CC_REQUIRE(precision == 2, "cc_gemm_bce_tc: bf16 dlogits come with bf16 operands (precision 2)");
     p.round_tf32 = 0;

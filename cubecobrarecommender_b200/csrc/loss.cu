@@ -471,6 +471,8 @@ softmax_kl_persistent_kernel(const float* __restrict__ z, int64_t ldz, const flo
 // Two launch shapes, chosen by the row length: 768 threads x 7 slots (85 registers per thread, 24 warps: rows of up to
 // 21 504 cards -- the 20 884 of the shipped checkpoints) and 512 threads x 11 slots (128 registers, 16 warps: up to 22 528).
 // More warps hide more of the shared-memory / MUFU latencies the kernel stalls on (ncu: profiles/r02/kl_regs_v1_stalls.txt).
+// GRAD = false (evaluation, cc_softmax_kl_loss): the kernel stops after sweep 2 -- row_loss / row_hit as with GRAD, no
+// dlogits, no column sums, nothing written back to shared memory; 8 bytes per element instead of 12.
 template <int WARPS>
 __device__ __forceinline__ float2 block_sum2_r(float a, float b, float2* red /* smem[WARPS] */) {
   a = warp_sum(a); b = warp_sum(b);
@@ -483,7 +485,7 @@ __device__ __forceinline__ float2 block_sum2_r(float a, float b, float2* red /* 
   return t;
 }
 
-template <bool FAST, int KLR_THREADS, int ITERS>
+template <bool FAST, int KLR_THREADS, int ITERS, bool GRAD = true>
 __global__ void __launch_bounds__(KLR_THREADS, 1)
 softmax_kl_regs_kernel(const float* __restrict__ z, int64_t ldz, const float* __restrict__ target, int64_t ldt,
                        const int32_t* __restrict__ target_rows, int32_t rows, int32_t num_cards, int32_t ncols_pad,
@@ -627,12 +629,19 @@ softmax_kl_regs_kernel(const float* __restrict__ z, int64_t ldz, const float* __
           else loss += tt[c] * (LOGF(tt[c]) - logq);
           sun += un ? tt[c] : 0.f;
         }
-        s4[i] = make_float4(ee[0], ee[1], ee[2], ee[3]);
-        tv[k] = make_float4(tt[0], tt[1], tt[2], tt[3]);
+        if constexpr (GRAD) {
+          s4[i] = make_float4(ee[0], ee[1], ee[2], ee[3]);
+          tv[k] = make_float4(tt[0], tt[1], tt[2], tt[3]);
+        }
       }
     }
-    const float2 ls = block_sum2_r<KLR_THREADS / 32>(loss, sun, red);
+    const float2 ls = block_sum2_r<KLR_THREADS / 32>(loss, GRAD ? sun : 0.f, red);
     if (threadIdx.x == 0) row_loss[r] = tlogt ? tlogt[trow] + double(ls.x) : double(ls.x);
+    if constexpr (!GRAD) {
+      __syncthreads();        // every thread is done with sz[buf] before the prefetch after next overwrites it
+      buf ^= 1;
+      continue;
+    }
     const float S = ls.y;
     const float qs = inv_sum * S * grad_scale;
     float4* d4 = dz16 ? nullptr : reinterpret_cast<float4*>(dz + int64_t(r) * lddz);
@@ -675,7 +684,7 @@ softmax_kl_regs_kernel(const float* __restrict__ z, int64_t ldz, const float* __
     __syncthreads();          // every thread is done with sz[buf] before the prefetch after next overwrites it
     buf ^= 1;
   }
-  if (dbias) {
+  if (GRAD && dbias) {
 #pragma unroll
     for (int k = 0; k < ITERS; ++k) {
       const int i = threadIdx.x + k * KLR_THREADS;
@@ -1073,6 +1082,41 @@ int cc_softmax_kl_fwd_bwd_metrics(const float* z, int64_t ldz, const float* targ
     softmax_kl_rows_kernel<false><<<rows, 1024, 0, st>>>(z, ldz, target, ldt, target_rows, num_cards, ncols_pad,
                                                          float(grad_scale), dz, lddz, row_loss, round_tf32);
   }
+  CC_CHECK_LAUNCH();
+  return CC_OK;
+}
+
+// Loss-only softmax-KL for evaluation: row_loss (and, with target_argmax, row_hit) exactly as
+// cc_softmax_kl_fwd_bwd_metrics computes them with the same tlogt and fast (= its round_tf32) flag; z is only read.
+// Register-resident kernel shapes only (num_cards % 4 == 0, num_cards <= 22 528, 16-byte aligned rows).
+int cc_softmax_kl_loss(const float* z, int64_t ldz, const float* target, int64_t ldt, const int32_t* target_rows,
+                       int32_t rows, int32_t num_cards, int32_t ncols_pad, const double* tlogt,
+                       const int32_t* target_argmax, double* row_loss, int32_t* row_hit, int fast, void* stream) {
+  CC_NVTX("cc_softmax_kl_loss");
+  CC_REQUIRE(z && target && row_loss, "cc_softmax_kl_loss: null pointer");
+  CC_REQUIRE(!target_argmax == !row_hit, "cc_softmax_kl_loss: target_argmax and row_hit are given together");
+  CC_REQUIRE(rows >= 0 && num_cards > 0 && ncols_pad >= num_cards, "cc_softmax_kl_loss: bad sizes");
+  auto fits = [&](int threads, int iters) { return (ncols_pad >> 2) <= (iters + 1) * threads && (num_cards >> 2) <= iters * threads; };
+  const bool fits768 = fits(768, 7) && g_kl_variant != 2, fits512 = fits(512, 11);
+  CC_REQUIRE(num_cards % 4 == 0 && ldz % 4 == 0 && ldt % 4 == 0 && ncols_pad % 4 == 0 && (fits768 || fits512) &&
+                 ((reinterpret_cast<uintptr_t>(z) | reinterpret_cast<uintptr_t>(target)) % 16 == 0),
+             "cc_softmax_kl_loss: num_cards %d outside the register kernel's shapes (num_cards %% 4 == 0, <= 22528, "
+             "16-byte aligned rows)", num_cards);
+  if (rows == 0) return CC_OK;
+  cudaStream_t st = as_stream(stream);
+  const size_t smem = size_t(num_cards) * 8;
+  const int grid = rows < sm_count() ? rows : sm_count();
+#define CC_KL_LOSS(FAST_, THREADS_, ITERS_)                                                                             \
+  do {                                                                                                                \
+    CC_CHECK_CUDA(cudaFuncSetAttribute(softmax_kl_regs_kernel<FAST_, THREADS_, ITERS_, false>,                        \
+                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                      \
+    softmax_kl_regs_kernel<FAST_, THREADS_, ITERS_, false><<<grid, THREADS_, smem, st>>>(                             \
+        z, ldz, target, ldt, target_rows, rows, num_cards, ncols_pad, 0.f, nullptr, 0, row_loss, 0, nullptr, nullptr, \
+        0, tlogt, target_argmax, row_hit);                                                                            \
+  } while (0)
+  if (fits768) { if (fast) CC_KL_LOSS(true, 768, 7); else CC_KL_LOSS(false, 768, 7); }
+  else         { if (fast) CC_KL_LOSS(true, 512, 11); else CC_KL_LOSS(false, 512, 11); }
+#undef CC_KL_LOSS
   CC_CHECK_LAUNCH();
   return CC_OK;
 }

@@ -28,6 +28,9 @@ KERAS_ADAM = dict(lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-7)
 # which CC_FIRST_LAYER values select the tensor-core first layer.  "auto" is in: measured on the B200 at B = 4096,
 # C = 20 884 (profiles/r02/ab_first_layer.txt): x W1 as a kind::tf32 GEMM 144 us against 225 us for the gather (bf16: 79 us)
 FIRST_LAYER_TENSOR_WHEN = ("tensor", "auto")
+# widest rows the loss-only softmax-KL kernel takes (cc_softmax_kl_loss: the register kernel's 512 x 11 shape); evaluation
+# of wider rows runs the training kernel into scratch
+KL_LOSS_MAX_CARDS = 22528
 
 
 def alias_table(p: np.ndarray, device):
@@ -37,6 +40,11 @@ def alias_table(p: np.ndarray, device):
     alias = np.empty(len(p), dtype=np.int32)
     call("cc_alias_build_host", ptr(p), len(p), ptr(prob), ptr(alias))
     return torch.from_numpy(prob).to(device), torch.from_numpy(alias).to(device)
+
+
+def _to_bf16(src, dst):
+    """fp32 (rows, cols) view -> bf16 matrix, on the current stream."""
+    call("cc_convert_f32_bf16", ptr(src), src.stride(0), ptr(dst), dst.stride(0), src.shape[0], src.shape[1], stream_ptr())
 
 
 def full_identity_shard(num_cards: int, rank: int = 0, world: int = 1):
@@ -324,15 +332,22 @@ class DAEEngine:
         self._fixed_reg_rows = True
 
     # -- the step -------------------------------------------------------------------
-    def forward_backward(self):
+    def _forward(self, rows=None, reg_rows=None, sums=None, metrics=False):
+        """The forward half of the step: layers, fused losses, accuracy counts.  Training (``rows`` None): logits become
+        dlogits and the output biases' gradients are written, as ``forward_backward`` needs them.  Evaluation: the first
+        ``rows`` cubes of the loaded batch against reg rows ``reg_rows[:rows]``, loss-only kernels (no dlogits, no
+        gradient), and [bce_sum, kl_sum, binary_hits, categorical_hits] added into the device float64 vector ``sums``.
+        Returns (launches, BCE partials, their count, reg_dbias_fused) for the training path."""
         s, B, R, T = self.store, self.B, self.R, self.B + self.R
+        ev = rows is not None
+        Bm = rows if ev else B              # main rows and reg rows this pass computes
+        Rm = min(rows, R) if ev else R
+        rr = reg_rows if ev else self.reg_rows
         big16 = self.big16
         pr = "tf32" if big16 else self.precision     # every layer but the 512 <-> C passes of the "bf16" mode
         tc = pr != "fp32"               # tensor-core modes: operands rounded to tf32 where produced
 
-        def to_bf16(src, dst):          # fp32 (rows, cols) view -> bf16 matrix
-            call("cc_convert_f32_bf16", ptr(src), src.stride(0), ptr(dst), dst.stride(0), src.shape[0], src.shape[1],
-                 stream_ptr())
+        to_bf16 = _to_bf16
         x = self._x
         P, G, W = s.p, s.g, s.w         # master params, grads, the copy of the kernels the GEMMs read
         n_launch = 0
@@ -352,17 +367,18 @@ class DAEEngine:
                 n_launch += 1
             with self._timed("fw1_gemm"):
                 if big16:
-                    gemm(self.x_dense[:, :self.C], self.w1_16, a1[:B], bias=P("encoder_e1/bias"), relu=True,
+                    gemm(self.x_dense[:Bm, :self.C], self.w1_16, a1[:Bm], bias=P("encoder_e1/bias"), relu=True,
                          precision="bf16", round_out=True)
                 else:
-                    gemm(self.x_dense[:, :self.C], W("encoder_e1/kernel"), a1[:B], bias=P("encoder_e1/bias"), relu=True,
+                    gemm(self.x_dense[:Bm, :self.C], W("encoder_e1/kernel"), a1[:Bm], bias=P("encoder_e1/bias"), relu=True,
                          precision=pr, round_out=True)
         else:
             with self._timed("bag_fwd"):
-                bag_fwd(P("encoder_e1/kernel"), x.idx, x.row_start, x.row_len, P("encoder_e1/bias"), a1[:B], round_tf32=tc)
+                bag_fwd(P("encoder_e1/kernel"), x.idx, x.row_start[:Bm], x.row_len[:Bm], P("encoder_e1/bias"), a1[:Bm],
+                        round_tf32=tc)
         n_launch += 1
         if R:
-            bag_fwd(P("encoder_e1/kernel"), self.reg_rows, self.reg_start, self.reg_len, P("encoder_e1/bias"), a1[B:],
+            bag_fwd(P("encoder_e1/kernel"), rr, self.reg_start[:Rm], self.reg_len[:Rm], P("encoder_e1/bias"), a1[B:B + Rm],
                     round_tf32=tc)
             n_launch += 1
         if self.small_chain:
@@ -388,9 +404,12 @@ class DAEEngine:
                      round_out=tc)
                 h_ = acts_[i]
             return 3
-        towers = [("main", self.a[3][:B], self.md, self.z1, B)]
+        rows_of = lambda bufs, n: [b_[:n] for b_ in bufs]
+        md, rd = rows_of(self.md, Bm), rows_of(self.rd, Rm)
+        md_bits, rd_bits = rows_of(self.md_bits, Bm), rows_of(self.rd_bits, Rm)
+        towers = [("main", self.a[3][:Bm], md, self.z1, Bm)]
         if R:
-            towers.append(("reg", self.a[3][B:], self.rd, self.z2, R))
+            towers.append(("reg", self.a[3][B:B + Rm], rd, self.z2, Rm))
         bce_rows, bce_n = self.row_bce, B
         main_stream = torch.cuda.current_stream(self.dev)
         if self.use_side and self._side is None:
@@ -404,25 +423,37 @@ class DAEEngine:
             fork.record(main_stream)                       # the shared encoder's output is complete
             with torch.cuda.stream(self._side):
                 self._side.wait_event(fork)
-                n_launch += dec_small_fwd(dec_names("reg"), self.a[3][B:], self.rd, self.rd_bits)
+                n_launch += dec_small_fwd(dec_names("reg"), self.a[3][B:B + Rm], rd, rd_bits)
                 join.record(self._side)
-        for prefix, h, acts, z, rows in towers:
+        if ev:
+            eb = self._eval_buffers()
+            if tc:
+                eb["part"].zero_()          # a partial batch covers fewer (tile, warp) slots than the last one
+                if metrics:
+                    eb["acc"].zero_()
+        for prefix, h, acts, z, nrows in towers:
             names = dec_names(prefix)
             if prefix == "reg" and reg_small_on_side:
                 main_stream.wait_event(join)
                 h = acts[2]
             else:
-                n_launch += dec_small_fwd(names, h, acts, self.md_bits if prefix == "main" else self.rd_bits)
+                n_launch += dec_small_fwd(names, h, acts, md_bits if prefix == "main" else rd_bits)
                 h = acts[2]
             if big16:                   # the 512-wide activation as a bf16 operand
-                h16 = self.md2_16 if prefix == "main" else self.rd2_16
+                h16 = (self.md2_16 if prefix == "main" else self.rd2_16)[:nrows]
                 to_bf16(h, h16)
                 n_launch += 1
             if tc and prefix == "main":
-                # fused 512 -> C layer + sigmoid-BCE: logits stay in TMEM, only dlogits are written
+                # fused 512 -> C layer + sigmoid-BCE: logits stay in TMEM, only dlogits are written (evaluation: nothing
+                # but the loss / accuracy partials)
                 from . import tensorcore
                 with self._timed("big_gemm"):       # the epilogue also reduces dlogits' columns into the bias gradient
-                    if big16:
+                    if ev:
+                        tensorcore.gemm_bce(h16 if big16 else h, self.w4_16["main"][:, :self.C] if big16 else W(names[3] + "/kernel"),
+                                            P(names[3] + "/bias"), self.y_bits[:Bm], float(Bm) * float(self.C), None,
+                                            eb["part"], precision="bf16" if big16 else pr, lddz=self.cpad,
+                                            acc_partial=eb["acc"] if metrics else None)
+                    elif big16:
                         tensorcore.gemm_bce(h16, self.w4_16["main"][:, :self.C], P(names[3] + "/bias"), self.y_bits,
                                             float(self.global_B) * float(self.C), self.dz1_16, self.bce_partial,
                                             precision="bf16", dbias=G(names[3] + "/bias"), acc_partial=self.acc_partial)
@@ -434,46 +465,128 @@ class DAEEngine:
             else:
                 with self._timed("big_gemm"):
                     if big16:
-                        gemm(h16, self.w4_16[prefix][:, :self.C], z[:, :self.C], bias=P(names[3] + "/bias"), precision="bf16")
+                        gemm(h16, self.w4_16[prefix][:, :self.C], z[:nrows, :self.C], bias=P(names[3] + "/bias"),
+                             precision="bf16")
                     else:
-                        gemm(h, W(names[3] + "/kernel"), z[:, :self.C], bias=P(names[3] + "/bias"), precision=pr)
+                        gemm(h, W(names[3] + "/kernel"), z[:nrows, :self.C], bias=P(names[3] + "/bias"), precision=pr)
             n_launch += 1
-        # ---------------- losses (logits -> dlogits in place) ----------------
+        # ---------------- losses (training: logits -> dlogits in place) ----------------
         if not tc:
-            if self.want_metrics:           # the exact-fp32 mode keeps its logits in memory: count before they become dlogits
-                call("cc_binary_accuracy_rows", ptr(self.z1), self.z1.stride(0), ptr(self.y_bits), self.yw, B, self.C,
-                     ptr(self.row_correct), st)
+            if ev:
+                if metrics:
+                    call("cc_binary_accuracy_rows", ptr(self.z1), self.z1.stride(0), ptr(self.y_bits), self.yw, Bm, self.C,
+                         ptr(eb["correct"]), st)
+                call("cc_bce_logits_fwd_bwd", ptr(self.z1), self.z1.stride(0), ptr(self.y_bits), self.yw, Bm, self.C,
+                     self.cpad, float(Bm) * float(self.C), None, 0, ptr(eb["bce"]), st)
+            else:
+                if self.want_metrics:       # the exact-fp32 mode keeps its logits in memory: count before they become dlogits
+                    call("cc_binary_accuracy_rows", ptr(self.z1), self.z1.stride(0), ptr(self.y_bits), self.yw, B, self.C,
+                         ptr(self.row_correct), st)
+                    n_launch += 1
+                with self._timed("bce"):
+                    call("cc_bce_logits_fwd_bwd", ptr(self.z1), self.z1.stride(0), ptr(self.y_bits), self.yw, B, self.C,
+                         self.cpad, float(self.global_B) * float(self.C), ptr(self.z1), self.z1.stride(0),
+                         ptr(self.row_bce), st)
                 n_launch += 1
-            with self._timed("bce"):
-                call("cc_bce_logits_fwd_bwd", ptr(self.z1), self.z1.stride(0), ptr(self.y_bits), self.yw, B, self.C,
-                     self.cpad, float(self.global_B) * float(self.C), ptr(self.z1), self.z1.stride(0),
-                     ptr(self.row_bce), st)
-            n_launch += 1
         reg_dbias_fused = False
         if R:
             # the persistent softmax-KL kernel also reduces dlogits' columns into the reg tower's output bias gradient
             reg_dbias_fused = bool(_lib.load().cc_softmax_kl_fuses_dbias(self.C, self.cpad, self.z2.stride(0),
                                                                          self.mhat.stride(0), self.z2.stride(0)))
+            want_hit = metrics if ev else self.want_metrics
+            row_kl, row_hit = (eb["kl"], eb["hit"]) if ev else (self.row_kl, self.row_hit)
             with self._timed("softmax_kl"):
-                if big16:
-                    if not reg_dbias_fused:
-                        raise RuntimeError("bf16 mode needs the persistent softmax-KL kernel (num_cards % 4 == 0, C <= 25600)")
-                    call("cc_softmax_kl_fwd_bwd_metrics", ptr(self.z2), self.z2.stride(0), ptr(self.mhat), self.mhat.stride(0),
-                         ptr(self.reg_rows), R, self.C, self.cpad, self.reg / float(self.global_R), None, 0,
-                         ptr(self.row_kl), 1, ptr(G(dec_names("reg")[3] + "/bias")), ptr(self.dz2_16),
-                         self.dz2_16.stride(0), ptr(self.kl_table()), ptr(self.kl_argmax()) if self.want_metrics else None,
-                         ptr(self.row_hit) if self.want_metrics else None, st)
+                if ev and self.C % 4 == 0 and self.C <= KL_LOSS_MAX_CARDS and self.mhat.stride(0) % 4 == 0:
+                    call("cc_softmax_kl_loss", ptr(self.z2), self.z2.stride(0), ptr(self.mhat), self.mhat.stride(0), ptr(rr),
+                         Rm, self.C, self.cpad, ptr(self.kl_table()), ptr(self.kl_argmax()) if want_hit else None,
+                         ptr(row_kl), ptr(row_hit) if want_hit else None, int(tc), st)
                 else:
-                    if self.want_metrics and not reg_dbias_fused:
-                        raise RuntimeError("metrics need the persistent softmax-KL kernel (num_cards % 4 == 0, C <= 25600)")
-                    call("cc_softmax_kl_fwd_bwd_metrics", ptr(self.z2), self.z2.stride(0), ptr(self.mhat), self.mhat.stride(0),
-                         ptr(self.reg_rows), R, self.C, self.cpad, self.reg / float(self.global_R), ptr(self.z2),
-                         self.z2.stride(0), ptr(self.row_kl), int(tc),
-                         ptr(G(dec_names("reg")[3] + "/bias")) if reg_dbias_fused else None, None, 0,
-                         ptr(self.kl_table()) if reg_dbias_fused else None,
-                         ptr(self.kl_argmax()) if self.want_metrics else None,
-                         ptr(self.row_hit) if self.want_metrics else None, st)
+                    # training; and evaluation of rows wider than the loss-only kernel takes: the training kernel with
+                    # its dlogits written over the (scratch) logits and its bias gradient into a scratch vector
+                    dbias = eb["dbias"] if ev else G(dec_names("reg")[3] + "/bias")
+                    if big16:
+                        if not reg_dbias_fused:
+                            raise RuntimeError("bf16 mode needs the persistent softmax-KL kernel (num_cards % 4 == 0, C <= 25600)")
+                        call("cc_softmax_kl_fwd_bwd_metrics", ptr(self.z2), self.z2.stride(0), ptr(self.mhat), self.mhat.stride(0),
+                             ptr(rr), Rm, self.C, self.cpad, self.reg / float(self.global_R), None, 0,
+                             ptr(row_kl), 1, ptr(dbias), ptr(self.dz2_16),
+                             self.dz2_16.stride(0), ptr(self.kl_table()), ptr(self.kl_argmax()) if want_hit else None,
+                             ptr(row_hit) if want_hit else None, st)
+                    else:
+                        if want_hit and not reg_dbias_fused:
+                            raise RuntimeError("metrics need the persistent softmax-KL kernel (num_cards % 4 == 0, C <= 25600)")
+                        call("cc_softmax_kl_fwd_bwd_metrics", ptr(self.z2), self.z2.stride(0), ptr(self.mhat), self.mhat.stride(0),
+                             ptr(rr), Rm, self.C, self.cpad, self.reg / float(self.global_R), ptr(self.z2),
+                             self.z2.stride(0), ptr(row_kl), int(tc),
+                             ptr(dbias) if reg_dbias_fused else None, None, 0,
+                             ptr(self.kl_table()) if reg_dbias_fused else None,
+                             ptr(self.kl_argmax()) if want_hit else None,
+                             ptr(row_hit) if want_hit else None, st)
             n_launch += 1
+        if ev:
+            sums[0] += (eb["part"] if tc else eb["bce"][:Bm]).sum()
+            if R:
+                sums[1] += eb["kl"][:Rm].sum()
+            if metrics:
+                sums[2] += (eb["acc"] if tc else eb["correct"][:Bm]).sum()
+                if R:
+                    sums[3] += eb["hit"][:Rm].sum()
+        return n_launch, bce_rows, bce_n, reg_dbias_fused
+
+    def _eval_buffers(self):
+        """Scratch of the evaluation pass (allocated on first use): BCE / accuracy partials of the loss-only GEMM,
+        per-row sums, and a bias-gradient sink for rows too wide for the loss-only KL kernel."""
+        if getattr(self, "_eval_bufs", None) is None:
+            d, f64 = self.dev, torch.float64
+            n_part = self.bce_partial.numel() if self.bce_partial is not None else 1
+            self._eval_bufs = dict(part=torch.zeros(n_part, dtype=f64, device=d), acc=torch.zeros(n_part, dtype=f64, device=d),
+                                   bce=torch.zeros(self.B, dtype=f64, device=d), correct=torch.zeros(self.B, dtype=f64, device=d),
+                                   kl=torch.zeros(max(self.R, 1), dtype=f64, device=d),
+                                   hit=torch.zeros(max(self.R, 1), dtype=torch.int32, device=d),
+                                   dbias=torch.zeros(self.C, dtype=torch.float32, device=d))
+        return self._eval_bufs
+
+    def sample_eval_batch(self, indptr, indices, batch_ids, alias_prob, alias_idx, noise, noise_std, seed, counter):
+        """Noise function F for ``len(batch_ids)`` (<= B) validation cubes, keyed by (seed, cube id, ``*counter``): the
+        caller holds the counter constant, so a cube gets the same corruption whenever it is evaluated.  Draws no reg
+        rows and advances no counter; overwrites the batch loaded by sample_batch / set_batch."""
+        self._check_no_prefetch()
+        n = int(batch_ids.numel())
+        if not 0 < n <= self.B:
+            raise ValueError(f"{n} validation cubes in a batch of an engine built for {self.B}")
+        call("cc_noise_ex", ptr(indptr), ptr(indices), ptr(batch_ids), n, self.C, ptr(alias_prob), ptr(alias_idx),
+             float(noise), float(noise_std), int(seed), ptr(counter), self.max_cube_size, self.x_stride, ptr(self.x_idx),
+             ptr(self.x_len), ptr(self.y_bits), self.yw, ptr(self.flips), ptr(self.overflow), ptr(self.x_dense),
+             self.cpad if self.x_dense is not None else 0, int(self.big16), stream_ptr())
+        self._x = SparseBatch(self.x_idx, self.x_start, self.x_len)
+
+    def evaluate_batch(self, rows, reg_rows, sums, metrics=True):
+        """Loss-only forward of the first ``rows`` cubes of the loaded batch, cube i paired with reg row ``reg_rows[i]``;
+        adds [bce_sum, kl_sum, binary_hits, categorical_hits] into ``sums`` (device float64 (4,)), no host sync.  Leaves
+        the parameters, gradients, tf32 shadow, Adam slots and both step counters untouched."""
+        self._check_no_prefetch()
+        rows = int(rows)
+        if not 0 < rows <= (min(self.B, self.R) if self.R else self.B):
+            raise ValueError(f"evaluate_batch: rows={rows} outside (0, {min(self.B, self.R) if self.R else self.B}]")
+        if self.R and reg_rows.numel() < rows:
+            raise ValueError("evaluate_batch: fewer reg rows than cubes")
+        self._forward(rows, reg_rows, sums, bool(metrics))
+
+    def _check_no_prefetch(self):
+        if self._prefetch_ready is not None:
+            raise RuntimeError("a batch prefetched by train_step(next_batch=...) is pending: evaluating now would overwrite it")
+
+    def forward_backward(self):
+        s, B, R = self.store, self.B, self.R
+        big16 = self.big16
+        pr = "tf32" if big16 else self.precision
+        tc = pr != "fp32"
+
+        to_bf16 = _to_bf16
+        x = self._x
+        P, G, W = s.p, s.g, s.w
+        main_stream = torch.cuda.current_stream(self.dev)
+        n_launch, bce_rows, bce_n, reg_dbias_fused = self._forward()
         side_used = [0]
 
         def on_side(fn):

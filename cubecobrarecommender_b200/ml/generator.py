@@ -18,10 +18,16 @@ as the NumPy array the reference exposes (one small D2H per epoch).
 """
 from __future__ import annotations
 
+import copy
+
 import numpy as np
 import torch
 
 from ..sparse import CubeCSR
+
+# validation noise: its own seed (the generator seed mixed with this salt) and a counter held at this value
+VALIDATION_SEED_SALT = 0x7A11DA7E
+VALIDATION_COUNTER = 0
 
 
 class DataGenerator:
@@ -53,6 +59,47 @@ class DataGenerator:
         self.indptr = torch.from_numpy(np.ascontiguousarray(self.csr.indptr)).to(self.device)
         self.indices_dev = torch.from_numpy(np.ascontiguousarray(self.csr.indices)).to(self.device)
         self._step = torch.zeros(1, dtype=torch.int64, device=self.device)
+        self._validation = None
+
+    def split(self, validation_split: float):
+        """``(train, val)`` generators: Keras' ``validation_split`` -- the validation cubes are the last
+        ``round(N_cubes * validation_split)`` cubes in CSR order, taken before any shuffling.  Both share this generator's
+        device M-hat, ``neg_sampler`` and alias table; each gets its own (small) device copy of its cubes."""
+        if not 0.0 < float(validation_split) < 1.0:
+            raise ValueError(f"validation_split must lie in (0, 1), got {validation_split}")
+        k_val = int(round(self.N_cubes * float(validation_split)))
+        if not 0 < k_val < self.N_cubes:
+            raise ValueError(f"validation_split {validation_split} of {self.N_cubes} cubes leaves an empty side")
+        self.mhat_device()                  # built once here, shared by both halves
+        cut = self.N_cubes - k_val
+        return self._subset(0, cut), self._subset(cut, self.N_cubes)
+
+    def _subset(self, lo, hi):
+        g = copy.copy(self)
+        g.csr = self.csr.rows(np.arange(lo, hi))
+        g.N_cubes = g.csr.num_cubes
+        g.indptr = torch.from_numpy(np.ascontiguousarray(g.csr.indptr)).to(self.device)
+        g.indices_dev = torch.from_numpy(np.ascontiguousarray(g.csr.indices)).to(self.device)
+        g._step = torch.zeros(1, dtype=torch.int64, device=self.device)
+        g._validation = None
+        g.reset_indices()
+        return g
+
+    def validation_draws(self):
+        """``(seed, counter, reg_rows)`` of this generator used as a validation set.  The noise kernel keys its draws by
+        (seed, cube id, counter): validation uses a seed of its own and a counter that never moves, so every cube gets
+        the same corruption in every epoch, whatever the batch size or the number of ranks -- epochs are comparable
+        (training redraws its noise every step).  ``reg_rows`` (device int32, one per cube) pairs validation cube v with
+        M-hat row ``reg_rows[v]``; drawn once."""
+        if getattr(self, "_validation", None) is None:
+            from .._lib import call, ptr, stream_ptr
+            seed = (self.seed * 0x9E3779B97F4A7C15 + VALIDATION_SEED_SALT) % (1 << 64)
+            counter = torch.full((1,), VALIDATION_COUNTER, dtype=torch.int64, device=self.device)
+            rows = torch.empty(max(self.N_cubes, 1), dtype=torch.int32, device=self.device)
+            call("cc_sample_reg_rows", ptr(self.alias_prob), ptr(self.alias_idx), self.N_cards, self.N_cubes,
+                 seed ^ 0x5DEECE66D, ptr(counter), ptr(rows), stream_ptr())
+            self._validation = (seed, counter, rows)
+        return self._validation
 
     def mhat_device(self, ld=None) -> torch.Tensor:
         """float32 M-hat on the device (what Keras would see after its float32 cast)."""

@@ -34,17 +34,20 @@ def gemm(a, b, c, *, transa=False, transb=False, bias=None, relu=False, mask=Non
     return c
 
 
-def gemm_bce(a, w, bias, ybits, count, dz, loss_partial, precision="tf32", round_out=True, dbias=None, acc_partial=None):
+def gemm_bce(a, w, bias, ybits, count, dz, loss_partial, precision="tf32", round_out=True, dbias=None, acc_partial=None,
+             lddz=None):
     """Fused  z = a @ w + bias -> BCE loss partials + dlogits  (z never stored); ``dbias`` (optional, float [n])
     receives the column sums of dlogits = the gradient of ``bias``; ``acc_partial`` (optional, float64 like
-    ``loss_partial``) the counts of correctly rounded cells (Keras binary_accuracy)."""
+    ``loss_partial``) the counts of correctly rounded cells (Keras binary_accuracy).  ``dz`` None: loss (and accuracy)
+    partials only, laid out for a dlogit matrix of row stride ``lddz``."""
     m, k = a.shape
     n = w.shape[1]
-    dz16 = dz.dtype == torch.bfloat16        # bf16 dlogits for the bf16 dW / dX GEMMs ("bf16" mode)
+    dz16 = dz is not None and dz.dtype == torch.bfloat16        # bf16 dlogits for the bf16 dW / dX GEMMs ("bf16" mode)
     if dz16 and precision != "bf16":
         raise TypeError("bf16 dlogits come with bf16 operands")
     call("cc_gemm_bce_tc_ex", PRECISION_CODE[precision], m, n, k, ptr(a), a.stride(0), ptr(w), w.stride(0), ptr(bias),
-         ptr(ybits), ybits.stride(0), float(count), ptr(dz), dz.stride(0), ptr(loss_partial), ptr(dbias),
+         ptr(ybits), ybits.stride(0), float(count), ptr(dz), dz.stride(0) if dz is not None else int(lddz),
+         ptr(loss_partial), ptr(dbias),
          int(round_out and precision == "tf32"), int(dz16), ptr(acc_partial), stream_ptr())
 
 

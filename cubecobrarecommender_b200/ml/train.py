@@ -1,6 +1,6 @@
 """Drop-in for reference ``src/ml/train.py``.
 
-    python -m cubecobrarecommender_b200.ml.train epochs batch_size name reg noise [seed]
+    python -m cubecobrarecommender_b200.ml.train epochs batch_size name reg noise [seed] [--validation-split F]
 
 Same positional arguments (reference train.py:28-38), same inputs (``data/maps/nameToId.json``,
 ``data/cube/*.json``, ``output/full_adj_mtx.npy``), same M-hat construction (train.py:69-71), loss and
@@ -26,8 +26,62 @@ def reset_random_seeds(seed):
     random.seed(seed)
 
 
+def progress_line(steps, seconds, logs):
+    """Keras' end-of-epoch progress line: ``steps/steps - Ns - key: value - ...`` in the order of ``logs``."""
+    return f"{steps}/{steps} - {seconds:.0f}s" + "".join(f" - {k}: {v:.4f}" for k, v in logs.items())
+
+
+def shard_range(n, rank, world):
+    """[lo, hi) of the contiguous shard of n items that rank ``rank`` of ``world`` takes (sizes differ by at most one)."""
+    return (n * rank) // world, (n * (rank + 1)) // world
+
+
+def evaluate(model, generator, reg, *, group=None, metrics=True, engine=None):
+    """Keras' ``model.evaluate(generator)``: ``{"loss", "output_1_loss", "output_2_loss", "output_1_accuracy",
+    "output_2_accuracy"}`` over every cube of ``generator``, as sample-weighted means over the whole set:
+    output_1_loss = sum BCE / (K C), output_2_loss = sum_v KL_v / K, loss = output_1_loss + reg * output_2_loss, the
+    accuracies = hits / (K C) and hits / K.  Cube v is corrupted by the generator's fixed validation noise and paired
+    with reg row v of its fixed draw (``DataGenerator.validation_draws``), so the result does not depend on the batch
+    size or the number of ranks beyond summation order.  Under ``torchrun`` each rank evaluates a contiguous shard of the
+    cubes and one all_reduce adds the sums.  ``engine``: a DAEEngine to run on (``fit`` passes its training engine);
+    none of its parameters, gradients, Adam slots or counters change.  Note that M-hat is built from every cube, the
+    held-out ones included."""
+    import torch.distributed as dist
+    from .engine import DAEEngine
+    world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
+    rank = dist.get_rank(group) if world > 1 else 0
+    k = generator.N_cubes
+    if k < 1:
+        raise ValueError("evaluate: the generator holds no cubes")
+    if engine is None:
+        lb = max(generator.batch_size // world, 1)
+        engine = DAEEngine(model, generator.mhat_device(), batch=lb, reg_rows=lb, reg=reg,
+                           max_cube_size=max(generator.csr.max_size, 1), group=group)
+    seed, counter, reg_rows = generator.validation_draws()
+    lo, hi = shard_range(k, rank, world)
+    step = min(engine.B, engine.R) if engine.R else engine.B
+    sums = torch.zeros(4, dtype=torch.float64, device=model.device)
+    ids = torch.arange(k, dtype=torch.int32, device=model.device)
+    for b0 in range(lo, hi, step):
+        b1 = min(b0 + step, hi)
+        engine.sample_eval_batch(generator.indptr, generator.indices_dev, ids[b0:b1], generator.alias_prob,
+                                 generator.alias_idx, generator.noise, generator.noise_std, seed, counter)
+        engine.evaluate_batch(b1 - b0, reg_rows[b0:b1], sums, metrics=metrics)
+    if world > 1:
+        dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
+    engine.check_overflow()
+    t = sums.cpu().numpy()
+    c = float(generator.N_cards)
+    bce, kl = t[0] / (k * c), t[1] / k
+    out = {"loss": float(bce + reg * kl), "output_1_loss": float(bce), "output_2_loss": float(kl)}
+    if metrics:
+        out.update({"output_1_accuracy": float(t[2] / (k * c)), "output_2_accuracy": float(t[3] / k)})
+    return out
+
+
 def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch=None, max_cube_size=None,
-        initial_epoch=0, checkpoint_dir=None, save_every=None, overflow_check_every=50, metrics=True):
+        initial_epoch=0, checkpoint_dir=None, save_every=None, overflow_check_every=50, metrics=True,
+        validation_data=None, validation_split=0.0, validation_freq=1):
     """``autoencoder.fit(generator, epochs=epochs)`` (reference train.py:99-102).  Returns the history
     ``[{"loss", "output_1_loss", "output_2_loss", "output_1_accuracy", "output_2_accuracy"}]`` per epoch (means over
     the epoch's steps, like Keras' progress line).  ``metrics`` mirrors ``compile(..., metrics=['accuracy'])`` (reference
@@ -37,7 +91,13 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
     Beyond the reference (SURVEY.md 8f-3): ``initial_epoch`` (Keras' own argument name) continues a run -- the epoch
     shuffle is a function of (seed, epoch), Adam's step counter lives in the model -- and every ``save_every`` epochs the
     model, its Adam slots and the number of completed epochs are written to ``checkpoint_dir`` (rank 0 writes; in p2p
-    data-parallel mode the sliced Adam slots are gathered first)."""
+    data-parallel mode the sliced Adam slots are gathered first).
+
+    Held-out validation, with Keras' semantics: ``validation_data`` (a DataGenerator) or ``validation_split`` (the last
+    fraction of the cubes, see ``DataGenerator.split``; ignored when ``validation_data`` is given) is evaluated (see
+    ``evaluate``) after every epoch with ``(epoch + 1) % validation_freq == 0``, and that epoch's history entry and
+    progress line gain ``val_loss``, ``val_output_1_loss``, ``val_output_2_loss`` and, with ``metrics``, the two
+    ``val_*_accuracy`` keys."""
     import torch.distributed as dist
     from .engine import DAEEngine
     world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
@@ -46,8 +106,14 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
     if gb % world:
         raise ValueError(f"batch_size {gb} must be divisible by the number of ranks {world}")
     lb = gb // world
+    val = validation_data
+    if val is None and validation_split:
+        generator, val = generator.split(validation_split)
+    if int(validation_freq) < 1:
+        raise ValueError(f"validation_freq must be >= 1, got {validation_freq}")
+    sizes = [generator.csr.max_size] + ([val.csr.max_size] if val is not None else [])
     eng = DAEEngine(model, generator.mhat_device(), batch=lb, reg_rows=lb, reg=reg,
-                    max_cube_size=max_cube_size or max(generator.csr.max_size, 1), global_batch=gb,
+                    max_cube_size=max_cube_size or max(max(sizes), 1), global_batch=gb,
                     global_reg_rows=gb, group=group, metrics=metrics)
     history = []
     nsteps = steps_per_epoch or len(generator)
@@ -70,13 +136,13 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
         eng.check_overflow()
         mean = (acc / max(nsteps, 1)).cpu().numpy()
         history.append({"loss": float(mean[2]), "output_1_loss": float(mean[0]), "output_2_loss": float(mean[1])})
-        line = (f"{nsteps}/{nsteps} - {time.time() - t0:.0f}s - loss: {mean[2]:.4f} - output_1_loss: {mean[0]:.4f} "
-                f"- output_2_loss: {mean[1]:.4f}")
         if metrics:
             mm = (macc / max(nsteps, 1)).cpu().numpy()
             history[-1].update({"output_1_accuracy": float(mm[0]), "output_2_accuracy": float(mm[1])})
-            line += f" - output_1_accuracy: {mm[0]:.4f} - output_2_accuracy: {mm[1]:.4f}"
-        log(line)
+        if val is not None and (epoch + 1) % int(validation_freq) == 0:
+            vlogs = evaluate(model, val, reg, group=group, metrics=metrics, engine=eng)
+            history[-1].update({"val_" + key: v for key, v in vlogs.items()})
+        log(progress_line(nsteps, time.time() - t0, history[-1]))
         generator.on_epoch_end()
         if checkpoint_dir and save_every and (epoch + 1) % save_every == 0 and epoch + 1 < epochs:
             eng.gather_adam_state()
@@ -86,27 +152,45 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
     return history
 
 
-def main(argv=None):
-    """``train.py epochs batch_size name reg noise [seed]`` (reference train.py:28-38), plus two optional flags the
-    reference does not have: ``--save-every N`` writes a checkpoint to ``ml_files/<name>`` every N epochs, ``--resume``
-    continues from the checkpoint found there (weights, Adam slots, step counter, completed epochs)."""
-    from ..non_ml import utils
-    from .generator import DataGenerator
-    from .model import CC_Recommender
-    args = list(sys.argv[1:] if argv is None else argv)
+def parse_args(argv):
+    """The reference's positional arguments ``epochs batch_size name reg noise [seed]`` and the optional flags."""
+    args = list(argv)
     resume = "--resume" in args
     if resume:
         args.remove("--resume")
-    save_every = None
-    if "--save-every" in args:
-        i = args.index("--save-every")
-        save_every = int(args[i + 1])
-        del args[i:i + 2]
-    epochs, batch_size, name = int(args[0]), int(args[1]), args[2]
-    reg, noise = float(args[3]), float(args[4])
-    seed = 0
-    if len(args) == 6:
-        seed = int(args[5])
+    flags = {"--save-every": None, "--validation-split": 0.0}
+    for flag in flags:
+        if flag in args:
+            i = args.index(flag)
+            if i + 1 >= len(args):
+                raise SystemExit(f"{flag} needs a value")
+            flags[flag] = args[i + 1]
+            del args[i:i + 2]
+    if len(args) < 5:
+        raise SystemExit("usage: train.py epochs batch_size name reg noise [seed] [--save-every N] [--resume] "
+                         "[--validation-split F]")
+    split = float(flags["--validation-split"])
+    if not 0.0 <= split < 1.0:
+        raise SystemExit(f"--validation-split must lie in [0, 1), got {split}")
+    return {"epochs": int(args[0]), "batch_size": int(args[1]), "name": args[2], "reg": float(args[3]),
+            "noise": float(args[4]), "seed": int(args[5]) if len(args) == 6 else 0, "seed_given": len(args) == 6,
+            "resume": resume, "save_every": int(flags["--save-every"]) if flags["--save-every"] is not None else None,
+            "validation_split": split}
+
+
+def main(argv=None):
+    """``train.py epochs batch_size name reg noise [seed]`` (reference train.py:28-38), plus optional flags the
+    reference does not have: ``--save-every N`` writes a checkpoint to ``ml_files/<name>`` every N epochs, ``--resume``
+    continues from the checkpoint found there (weights, Adam slots, step counter, completed epochs),
+    ``--validation-split F`` holds the last fraction F of the cubes out of training and reports ``val_*`` losses and
+    accuracies on them after every epoch."""
+    from ..non_ml import utils
+    from .generator import DataGenerator
+    from .model import CC_Recommender
+    opts = parse_args(sys.argv[1:] if argv is None else argv)
+    epochs, batch_size, name, reg, noise, seed = (opts[k] for k in ("epochs", "batch_size", "name", "reg", "noise", "seed"))
+    resume, save_every = opts["resume"], opts["save_every"]
+    if opts["seed_given"]:
         reset_random_seeds(seed)
     import torch.distributed as dist
     if "RANK" in os.environ and int(os.environ.get("WORLD_SIZE", "1")) > 1:
@@ -135,7 +219,8 @@ def main(argv=None):
     else:
         autoencoder = CC_Recommender(num_cards, device="cuda", seed=seed, precision=precision)
     generator = DataGenerator(y_mtx, cubes, batch_size=batch_size, noise=noise, seed=seed)
-    fit(autoencoder, generator, epochs, reg, initial_epoch=initial_epoch, checkpoint_dir=dest, save_every=save_every)
+    fit(autoencoder, generator, epochs, reg, initial_epoch=initial_epoch, checkpoint_dir=dest, save_every=save_every,
+        validation_split=opts["validation_split"])
     if not dist.is_initialized() or dist.get_rank() == 0:
         autoencoder.save(dest, epoch=epochs)
     if dist.is_initialized():

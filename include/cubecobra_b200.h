@@ -210,7 +210,9 @@ int cc_gemm_tc(int precision, int transa, int transb, int m, int n, int k, const
  * float64 [cc_gemm_bce_partial_count(m, lddz)] holds per-(tile, warp) loss sums for cc_loss_finalize.  dbias (nullable,
  * float [n]) receives the column sums of dz, i.e. the gradient of the layer's bias (zeroed, then accumulated with float
  * atomics by the epilogue: summation order, hence the last bits, can differ between runs).  dz_bf16 != 0 (precision 2
- * only): dz is a bf16 matrix (lddz in elements), the form the bf16 dW / dX GEMMs consume. */
+ * only): dz is a bf16 matrix (lddz in elements), the form the bf16 dW / dX GEMMs consume.  dz == NULL: loss only
+ * (evaluation) -- the same partials, nothing else written; lddz still sizes loss_partial, and dbias must be NULL and
+ * dz_bf16 0 (anything else is rejected). */
 int cc_gemm_bce_tc(int precision, int m, int n, int k, const void* a, int64_t lda, const void* w, int64_t ldw,
                    const float* bias, const uint32_t* ybits, int64_t ywords, double count, void* dz, int64_t lddz,
                    double* loss_partial, float* dbias, int round_tf32, int dz_bf16, void* stream);
@@ -308,6 +310,13 @@ int cc_softmax_kl_fwd_bwd_metrics(const float* z, int64_t ldz, const float* targ
                                   int64_t lddz_bf16, const double* tlogt, const int32_t* target_argmax, int32_t* row_hit,
                                   void* stream);
 int cc_kl_target_argmax(const float* target, int64_t ldt, int32_t target_rows, int32_t num_cards, int32_t* out, void* stream);
+/* Loss only (evaluation): row_loss[r] and, with target_argmax, row_hit[r] (the two are nullable together), computed
+ * exactly as cc_softmax_kl_fwd_bwd_metrics computes them with the same tlogt (nullable) and fast (its round_tf32); no
+ * dlogits, no bias gradient, z is only read.  The register-resident kernel's shapes only (num_cards % 4 == 0, at most
+ * 22 528 cards, 16-byte aligned rows): anything else returns CC_ERR_ARGUMENT. */
+int cc_softmax_kl_loss(const float* z, int64_t ldz, const float* target, int64_t ldt, const int32_t* target_rows,
+                       int32_t rows, int32_t num_cards, int32_t ncols_pad, const double* tlogt,
+                       const int32_t* target_argmax, double* row_loss, int32_t* row_hit, int fast, void* stream);
 /* Which persistent kernel serves dbias != NULL: 0 = choose (512 threads with the target row and the column sums in
  * registers when num_cards <= 22 528, else the 1024-thread form), 1 = always the 1024-thread form (tests, A/B runs). */
 int cc_softmax_kl_set_variant(int variant);
