@@ -106,6 +106,65 @@ __device__ __forceinline__ float4 ld_nc_f4(const void* p) {
                : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
   return r;
 }
+// ---- the recommender's total order on (score, index): every select and the target-rank kernel ----------
+template <typename T> struct KeyOf;
+template <> struct KeyOf<float> {
+  using U = uint32_t; using K = unsigned long long; static constexpr int BITS = 64;
+  __device__ static U ord(float v) { v += 0.0f; U b = __float_as_uint(v); return b ^ ((b >> 31) ? 0xffffffffu : 0x80000000u); }
+};
+template <> struct KeyOf<double> {
+  using U = unsigned long long; using K = unsigned __int128; static constexpr int BITS = 96;
+  __device__ static U ord(double v) {
+    v += 0.0; U b = (U)__double_as_longlong(v);
+    return b ^ ((b >> 63) ? 0xffffffffffffffffull : 0x8000000000000000ull);
+  }
+};
+
+// composite key: (orderable score, tie word); all keys of one cube are distinct, so the
+// n-th largest is unique and {key >= it} has exactly n members.
+//   descending: larger score first, ties -> larger index first  (argsort(stable)[::-1])
+//   ascending : smaller score first, ties -> smaller index first (argsort(stable))
+template <typename T>
+__device__ __forceinline__ typename KeyOf<T>::K make_key(T v, uint32_t idx, int descending) {
+  using KO = KeyOf<T>;
+  typename KO::U u = KO::ord(v);
+  uint32_t t = idx;
+  if (!descending) { u = ~u; t = ~idx; }
+  return (typename KO::K(u) << 32) | typename KO::K(t);
+}
+
+// a bound on the RAW value such that no element whose key is >= thr fails `pass`: the threshold's own score, or --
+// fused sigmoid -- its logit.  The logit is evaluated in float32 (one thread computes it while the CTA waits, and a
+// double-precision log costs that thread several hundred cycles).  The probability is first moved 2e-6 relative to the
+// safe side (16-33 float32 ulps: covers the <= 3 ulp error of sigmoid_f32 = 1 / (1 + expf(-z)) with IEEE division, and
+// keeps 1 - p >= 2e-6); the float32 logit of the moved probability is then moved by a bound on its own evaluation error:
+// 1e-5 (1 + |L|) for the quotient and logf (~80 ulps of L) plus 2.5e-7 / (1 - p) for the rounding of p next to 1 (half
+// an ulp of p is 3e-8 of the 1 - p it is subtracted from).  A constant slack of 0.08 (round 1) was safe but let EVERY
+// element of a row whose logits lie within 0.08 of each other (an untrained model) into the survivor buffer, sending
+// the cube through the overflow path; the slack here is 1e-5 for logits near 0 and grows to 0.125 only where the sigmoid
+// saturates.  A looser bound only lets a few more elements into the survivor buffer; it never loses one (checked densely
+// against float32 sigmoid on the host, tests/test_rowselect_model.py).
+__device__ __forceinline__ float rs_logit_slack(float logit, float one_minus_p) {
+  return 1e-5f * (1.f + fabsf(logit)) + 2.5e-7f / one_minus_p;
+}
+template <bool SIGMOID>
+__device__ __forceinline__ float rs_raw_bound(unsigned long long thr, int descending) {
+  if (thr == 0ull) return descending ? -INFINITY : INFINITY;
+  uint32_t u = (uint32_t)(thr >> 32);
+  if (!descending) u = ~u;
+  const float pthr = __uint_as_float((u & 0x80000000u) ? (u ^ 0x80000000u) : ~u);
+  if (!SIGMOID) return pthr;
+  if (descending) {
+    const float pm = pthr * (1.f - 2e-6f) - 1e-37f;
+    if (pm <= 0.f) return -INFINITY;
+    const float l = logf(pm / (1.f - pm));
+    return l - rs_logit_slack(l, 1.f - pm);
+  }
+  const float pp = pthr * (1.f + 2e-6f) + 1e-37f;
+  if (pp >= 1.f) return INFINITY;
+  const float l = logf(pp / (1.f - pp));
+  return l + rs_logit_slack(l, 1.f - pp);
+}
 #endif
 
 }  // namespace cc

@@ -221,6 +221,22 @@ def topn_masked(scores: torch.Tensor, mask_ptr: torch.Tensor, mask_idx: torch.Te
     return ids, vals, cnt
 
 
+def rank_targets(scores: torch.Tensor, mask_ptr: torch.Tensor, mask_idx: torch.Tensor, target_ptr: torch.Tensor,
+                 target_idx: torch.Tensor, *, sigmoid=False, out=None) -> torch.Tensor:
+    """int32 rank of every target entry (cc_rank_targets_f32): the 0-based slot at which the descending
+    :func:`topn_masked` select over the cards not listed in the mask row would return it, or -1 for a target that is
+    masked or out of range.  ``scores`` float32 (batch, >= C) with unit column stride, C = ``scores.shape[1]``;
+    ``sigmoid=True``: ``scores`` are logits, ranked by their float32 sigmoid.  ``out``: int32, one entry per
+    ``target_idx`` entry (default: allocated)."""
+    if scores.dtype != torch.float32 or scores.dim() != 2 or scores.stride(1) != 1:
+        raise TypeError("scores must be a float32 (batch, C) tensor with unit column stride")
+    if out is None:
+        out = torch.empty(target_idx.numel(), dtype=torch.int32, device=scores.device)
+    call("cc_rank_targets_f32", ptr(scores), scores.stride(0), int(scores.shape[1]), int(scores.shape[0]),
+         ptr(mask_ptr), ptr(mask_idx), ptr(target_ptr), ptr(target_idx), int(sigmoid), ptr(out), stream_ptr())
+    return out
+
+
 class GraphRecommender:
     """M resident in HBM (float64); batched ``simple_recs`` / ``simple_cuts``."""
 

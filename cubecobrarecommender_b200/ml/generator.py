@@ -60,6 +60,7 @@ class DataGenerator:
         self.indices_dev = torch.from_numpy(np.ascontiguousarray(self.csr.indices)).to(self.device)
         self._step = torch.zeros(1, dtype=torch.int64, device=self.device)
         self._validation = None
+        self._holdout = None
 
     def split(self, validation_split: float):
         """``(train, val)`` generators: Keras' ``validation_split`` -- the validation cubes are the last
@@ -82,6 +83,7 @@ class DataGenerator:
         g.indices_dev = torch.from_numpy(np.ascontiguousarray(g.csr.indices)).to(self.device)
         g._step = torch.zeros(1, dtype=torch.int64, device=self.device)
         g._validation = None
+        g._holdout = None
         g.reset_indices()
         return g
 
@@ -100,6 +102,19 @@ class DataGenerator:
                  seed ^ 0x5DEECE66D, ptr(counter), ptr(rows), stream_ptr())
             self._validation = (seed, counter, rows)
         return self._validation
+
+    def holdout_split(self, fraction: float):
+        """``(visible, hidden, evaluated)`` of ``ranking.holdout_split`` over this generator's cubes, with a seed of its
+        own (the generator seed mixed with ``ranking.HOLDOUT_SEED_SALT``): computed once per fraction on the host, so
+        every epoch hides the same cards, and no random stream of the generator is drawn from."""
+        from .ranking import HOLDOUT_SEED_SALT, holdout_split
+        if self._holdout is None:
+            self._holdout = {}
+        fraction = float(fraction)
+        if fraction not in self._holdout:
+            seed = (self.seed * 0x9E3779B97F4A7C15 + HOLDOUT_SEED_SALT) % (1 << 64)
+            self._holdout[fraction] = holdout_split(self.csr, fraction, seed)
+        return self._holdout[fraction]
 
     def mhat_device(self, ld=None) -> torch.Tensor:
         """float32 M-hat on the device (what Keras would see after its float32 cast)."""

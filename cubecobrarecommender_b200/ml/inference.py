@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from .._lib import call, ptr, stream_ptr
-from ..graph import topn_masked
+from ..graph import rank_targets, topn_masked
 from ..sparse import CubeCSR
 from .model import CC_Recommender, SparseBatch
 
@@ -42,6 +42,47 @@ class MLRecommender:
 
     FUSED_MAX_N = 128        # cc_topn_masked_sigmoid_f32's limit (warp-per-cube streaming select)
 
+    def _forward_chunks(self, csr: CubeCSR, *others: CubeCSR):
+        """The chunked forward of ``recommend_device`` and ``target_ranks_device``: yields ``(lo, hi, idx, ptr_, z,
+        rest)`` per chunk of ``self.chunk`` cubes, where ``idx`` / ``ptr_`` are rows [lo, hi) of ``csr`` on the device,
+        ``z`` the (hi - lo, C) logits of ``decoder(encoder(rows))`` and ``rest`` one ``(idx, ptr)`` device pair of rows
+        [lo, hi) per CSR in ``others``.  Chunk i+1's rows are uploaded on a copy stream while chunk i computes; nothing
+        synchronises with the host."""
+        m = self.model
+        dev = m.device
+        k = csr.num_cubes
+        host = [(np.ascontiguousarray(c.indptr, dtype=np.int64), np.ascontiguousarray(c.indices, dtype=np.int32))
+                for c in (csr,) + others]
+        compute = torch.cuda.current_stream(dev)
+        copier = self._copy_stream = getattr(self, "_copy_stream", None) or torch.cuda.Stream(device=dev)
+
+        def upload(lo):
+            hi = min(lo + self.chunk, k)
+            parts = []
+            with torch.cuda.stream(copier):
+                for ip, ix in host:
+                    rows_h = ix[ip[lo]:ip[hi]]
+                    idx = torch.from_numpy(rows_h if len(rows_h) else np.zeros(1, np.int32)).to(dev, non_blocking=True)
+                    ptr_ = torch.from_numpy(ip[lo:hi + 1] - ip[lo]).to(dev, non_blocking=True)
+                    parts.append((idx, ptr_))
+                ev = torch.cuda.Event()
+                ev.record(copier)
+            for pair in parts:
+                for t in pair:
+                    t.record_stream(compute)       # allocated on the copy stream, consumed on the compute stream
+            return lo, hi, parts, ev
+
+        nxt = upload(0) if k else None
+        while nxt is not None:
+            lo, hi, parts, ev = nxt
+            nxt = upload(hi) if hi < k else None   # overlaps this chunk's kernels
+            compute.wait_event(ev)
+            idx, ptr_ = parts[0]
+            row_len = (ptr_[1:] - ptr_[:-1]).to(torch.int32)
+            sb = SparseBatch(idx, ptr_[:-1], row_len)
+            z = m._decode(m._encode(sb), "main")
+            yield lo, hi, idx, ptr_, z, parts[1:]
+
     def recommend_device(self, csr: CubeCSR, amount: int, want_cuts: bool = False):
         """The cubes run through encoder, decoder and the masked select in chunks of ``self.chunk`` with NO host
         synchronisation in between; chunk i+1's CSR rows are uploaded on a copy stream while chunk i computes, and
@@ -53,35 +94,12 @@ class MLRecommender:
         k = csr.num_cubes
         n = max(1, min(int(amount), csr.num_cards))
         ip = np.ascontiguousarray(csr.indptr, dtype=np.int64)
-        ix = np.ascontiguousarray(csr.indices, dtype=np.int32)
         ids = torch.empty((k, n), dtype=torch.int32, device=dev)
         vals = torch.empty((k, n), dtype=torch.float32, device=dev)
         cnts = torch.empty(k, dtype=torch.int32, device=dev)
         cuts = torch.empty(max(int(ip[-1]), 1), dtype=torch.float32, device=dev) if want_cuts else None
         fused = n <= self.FUSED_MAX_N
-        compute = torch.cuda.current_stream(dev)
-        copier = self._copy_stream = getattr(self, "_copy_stream", None) or torch.cuda.Stream(device=dev)
-
-        def upload(lo):
-            hi = min(lo + self.chunk, k)
-            rows_h = ix[ip[lo]:ip[hi]]
-            with torch.cuda.stream(copier):
-                idx = torch.from_numpy(rows_h if len(rows_h) else np.zeros(1, np.int32)).to(dev, non_blocking=True)
-                ptr_ = torch.from_numpy(ip[lo:hi + 1] - ip[lo]).to(dev, non_blocking=True)
-                ev = torch.cuda.Event()
-                ev.record(copier)
-            for t in (idx, ptr_):
-                t.record_stream(compute)           # allocated on the copy stream, consumed on the compute stream
-            return lo, hi, idx, ptr_, ev
-
-        nxt = upload(0) if k else None
-        while nxt is not None:
-            lo, hi, idx, ptr_, ev = nxt
-            nxt = upload(hi) if hi < k else None   # overlaps this chunk's kernels
-            compute.wait_event(ev)
-            row_len = (ptr_[1:] - ptr_[:-1]).to(torch.int32)
-            sb = SparseBatch(idx, ptr_[:-1], row_len)
-            z = m._decode(m._encode(sb), "main")
+        for lo, hi, idx, ptr_, z, _ in self._forward_chunks(csr):
             out = (ids[lo:hi], vals[lo:hi], cnts[lo:hi])
             if fused:    # sigmoid applied inside the select: the probability rows are never written
                 topn_masked(z, ptr_, idx, n, sigmoid=True, out=out)
@@ -95,6 +113,23 @@ class MLRecommender:
         if want_cuts:
             return ids, vals, cnts, cuts[:int(ip[-1])]
         return ids, vals, cnts
+
+    def target_ranks_device(self, visible: CubeCSR, hidden: CubeCSR) -> torch.Tensor:
+        """Leave-k-out ranks, int32 aligned with ``hidden.indices``, on the device.  Cube b's ``visible`` cards are the
+        model input and the mask; each of its ``hidden`` cards gets the 0-based slot at which ``recommend_device``
+        would list it (for any ``amount``), or -1 if it is also visible.  Same chunked pipeline as ``recommend_device``
+        with no host synchronisation; the ranks come from cc_rank_targets_f32 on the logits with the sigmoid fused
+        in, so no probability row is written."""
+        if hidden.num_cubes != visible.num_cubes or hidden.num_cards != visible.num_cards:
+            raise ValueError("visible and hidden must hold the same cubes over the same cards")
+        if visible.num_cards != self.model.N:
+            raise ValueError(f"the cubes span {visible.num_cards} cards, the model {self.model.N}")
+        hp = np.ascontiguousarray(hidden.indptr, dtype=np.int64)
+        ranks = torch.empty(max(int(hp[-1]), 1), dtype=torch.int32, device=self.model.device)
+        for lo, hi, idx, ptr_, z, ((t_idx, t_ptr),) in self._forward_chunks(visible, hidden):
+            if hp[hi] > hp[lo]:
+                rank_targets(z, ptr_, idx, t_ptr, t_idx, sigmoid=True, out=ranks[int(hp[lo]):int(hp[hi])])
+        return ranks[:int(hp[-1])]
 
     def recommend(self, csr: CubeCSR, amount: int, copy: bool = True, want_cuts: bool = False):
         """Returns (add_ids int32 (K, n), add_scores float32 (K, n), counts int32 (K,)) on the host.  Pass a

@@ -1,6 +1,7 @@
 """Drop-in for reference ``src/ml/train.py``.
 
     python -m cubecobrarecommender_b200.ml.train epochs batch_size name reg noise [seed] [--validation-split F]
+                                                 [--rank-at K1,K2,...]
 
 Same positional arguments (reference train.py:28-38), same inputs (``data/maps/nameToId.json``,
 ``data/cube/*.json``, ``output/full_adj_mtx.npy``), same M-hat construction (train.py:69-71), loss and
@@ -79,9 +80,47 @@ def evaluate(model, generator, reg, *, group=None, metrics=True, engine=None):
     return out
 
 
+def evaluate_recommendations(model, generator, *, at=(10, 50), holdout=0.2, group=None):
+    """Leave-k-out ranking quality of the recommendations over every cube of ``generator``: each cube of s >= 2 cards
+    hides ``min(s - 1, max(1, floor(holdout * s + 0.5)))`` of them (``DataGenerator.holdout_split``: the same cards in
+    every call), the model sees the rest, and every hidden card is ranked among all the cards the cube does not show,
+    in the order ``MLRecommender.recommend_device`` lists them.  Returns ``{"recall_at_k", "ndcg_at_k",
+    "hit_rate_at_k"}`` for each k in ``at``, ``"mrr"``, ``"mpr"`` (mean percentile rank: 0.5 for a random ranking) --
+    each a mean over the evaluated cubes, see ``ranking.ranking_sums`` -- plus ``"cubes"`` (evaluated) and ``"skipped"``
+    (fewer than two cards).  Under ``torchrun`` each rank takes a contiguous shard of the cubes and one all_reduce adds
+    the sums; the only host read is the final one.  Parameters, gradients, the tf32 shadow, Adam slots and step
+    counters are left untouched, and no random stream is drawn from.  M-hat is built from every cube, the held-out
+    ones included."""
+    import torch.distributed as dist
+    from .inference import MLRecommender
+    from .ranking import metric_names, ranking_sums
+    at = tuple(int(k) for k in at)
+    if not at or min(at) < 1:
+        raise ValueError(f"evaluate_recommendations: every k in `at` must be >= 1, got {at}")
+    world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
+    rank = dist.get_rank(group) if world > 1 else 0
+    k = generator.N_cubes
+    if k < 1:
+        raise ValueError("evaluate_recommendations: the generator holds no cubes")
+    visible, hidden, _ = generator.holdout_split(holdout)
+    vis, hid = visible.shard(rank, world), hidden.shard(rank, world)          # the cubes of shard_range(k, rank, world)
+    dev = model.device
+    ranks = MLRecommender(model).target_ranks_device(vis, hid)
+    hp = torch.from_numpy(np.ascontiguousarray(hid.indptr, dtype=np.int64)).to(dev, non_blocking=True)
+    n_cand = torch.from_numpy(generator.N_cards - np.diff(vis.indptr)).to(dev, non_blocking=True)
+    sums = ranking_sums(ranks, hp, n_cand, at)
+    if world > 1:
+        dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
+    t = sums.cpu().numpy()
+    cubes = int(round(t[0]))
+    out = {name: float(v / cubes) if cubes else float("nan") for name, v in zip(metric_names(at), t[1:])}
+    out.update({"cubes": cubes, "skipped": k - cubes})
+    return out
+
+
 def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch=None, max_cube_size=None,
         initial_epoch=0, checkpoint_dir=None, save_every=None, overflow_check_every=50, metrics=True,
-        validation_data=None, validation_split=0.0, validation_freq=1):
+        validation_data=None, validation_split=0.0, validation_freq=1, ranking_at=None, ranking_holdout=0.2):
     """``autoencoder.fit(generator, epochs=epochs)`` (reference train.py:99-102).  Returns the history
     ``[{"loss", "output_1_loss", "output_2_loss", "output_1_accuracy", "output_2_accuracy"}]`` per epoch (means over
     the epoch's steps, like Keras' progress line).  ``metrics`` mirrors ``compile(..., metrics=['accuracy'])`` (reference
@@ -97,9 +136,17 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
     fraction of the cubes, see ``DataGenerator.split``; ignored when ``validation_data`` is given) is evaluated (see
     ``evaluate``) after every epoch with ``(epoch + 1) % validation_freq == 0``, and that epoch's history entry and
     progress line gain ``val_loss``, ``val_output_1_loss``, ``val_output_2_loss`` and, with ``metrics``, the two
-    ``val_*_accuracy`` keys."""
+    ``val_*_accuracy`` keys.  ``ranking_at`` (a sequence of k): the same epochs also run ``evaluate_recommendations``
+    on the validation cubes with ``holdout=ranking_holdout`` and add ``val_recall_at_k``, ``val_ndcg_at_k`` and
+    ``val_hit_rate_at_k`` per k, ``val_mrr`` and ``val_mpr``."""
     import torch.distributed as dist
     from .engine import DAEEngine
+    if ranking_at is not None:
+        ranking_at = tuple(int(k) for k in ranking_at)
+        if validation_data is None and not validation_split:
+            raise ValueError("ranking_at needs validation data (validation_data or validation_split)")
+        if not ranking_at or min(ranking_at) < 1:
+            raise ValueError(f"every k in ranking_at must be >= 1, got {ranking_at}")
     world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
     rank = dist.get_rank(group) if world > 1 else 0
     gb = generator.batch_size
@@ -142,6 +189,9 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
         if val is not None and (epoch + 1) % int(validation_freq) == 0:
             vlogs = evaluate(model, val, reg, group=group, metrics=metrics, engine=eng)
             history[-1].update({"val_" + key: v for key, v in vlogs.items()})
+            if ranking_at is not None:
+                rlogs = evaluate_recommendations(model, val, at=ranking_at, holdout=ranking_holdout, group=group)
+                history[-1].update({"val_" + key: v for key, v in rlogs.items() if key not in ("cubes", "skipped")})
         log(progress_line(nsteps, time.time() - t0, history[-1]))
         generator.on_epoch_end()
         if checkpoint_dir and save_every and (epoch + 1) % save_every == 0 and epoch + 1 < epochs:
@@ -158,7 +208,7 @@ def parse_args(argv):
     resume = "--resume" in args
     if resume:
         args.remove("--resume")
-    flags = {"--save-every": None, "--validation-split": 0.0}
+    flags = {"--save-every": None, "--validation-split": 0.0, "--rank-at": None}
     for flag in flags:
         if flag in args:
             i = args.index(flag)
@@ -168,14 +218,24 @@ def parse_args(argv):
             del args[i:i + 2]
     if len(args) < 5:
         raise SystemExit("usage: train.py epochs batch_size name reg noise [seed] [--save-every N] [--resume] "
-                         "[--validation-split F]")
+                         "[--validation-split F] [--rank-at K1,K2,...]")
     split = float(flags["--validation-split"])
     if not 0.0 <= split < 1.0:
         raise SystemExit(f"--validation-split must lie in [0, 1), got {split}")
+    rank_at = None
+    if flags["--rank-at"] is not None:
+        try:
+            rank_at = tuple(int(v) for v in flags["--rank-at"].split(","))
+        except ValueError:
+            raise SystemExit(f"--rank-at takes comma-separated integers, got {flags['--rank-at']!r}") from None
+        if min(rank_at) < 1:
+            raise SystemExit(f"--rank-at values must be >= 1, got {flags['--rank-at']}")
+        if split == 0.0:
+            raise SystemExit("--rank-at ranks the held-out cubes: it needs --validation-split F")
     return {"epochs": int(args[0]), "batch_size": int(args[1]), "name": args[2], "reg": float(args[3]),
             "noise": float(args[4]), "seed": int(args[5]) if len(args) == 6 else 0, "seed_given": len(args) == 6,
             "resume": resume, "save_every": int(flags["--save-every"]) if flags["--save-every"] is not None else None,
-            "validation_split": split}
+            "validation_split": split, "rank_at": rank_at}
 
 
 def main(argv=None):
@@ -183,7 +243,8 @@ def main(argv=None):
     reference does not have: ``--save-every N`` writes a checkpoint to ``ml_files/<name>`` every N epochs, ``--resume``
     continues from the checkpoint found there (weights, Adam slots, step counter, completed epochs),
     ``--validation-split F`` holds the last fraction F of the cubes out of training and reports ``val_*`` losses and
-    accuracies on them after every epoch."""
+    accuracies on them after every epoch, ``--rank-at 10,50`` adds the leave-k-out ranking metrics of those cubes
+    (``val_recall_at_10``, ``val_ndcg_at_10``, ``val_hit_rate_at_10``, ..., ``val_mrr``, ``val_mpr``)."""
     from ..non_ml import utils
     from .generator import DataGenerator
     from .model import CC_Recommender
@@ -220,7 +281,7 @@ def main(argv=None):
         autoencoder = CC_Recommender(num_cards, device="cuda", seed=seed, precision=precision)
     generator = DataGenerator(y_mtx, cubes, batch_size=batch_size, noise=noise, seed=seed)
     fit(autoencoder, generator, epochs, reg, initial_epoch=initial_epoch, checkpoint_dir=dest, save_every=save_every,
-        validation_split=opts["validation_split"])
+        validation_split=opts["validation_split"], ranking_at=opts["rank_at"])
     if not dist.is_initialized() or dist.get_rank() == 0:
         autoencoder.save(dest, epoch=epochs)
     if dist.is_initialized():

@@ -142,6 +142,17 @@ int cc_topn_rowselect_profile(const float* logits, int64_t ld, int32_t num_cards
  * the float32 sigmoid when apply_sigmoid != 0 (scores are logits then).  out: float32 [row_ptr[batch]]. */
 int cc_cuts_gather_f32(const float* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* row_ptr,
                        const int32_t* idx, int apply_sigmoid, float* out, void* stream);
+/* Target ranks for leave-k-out evaluation.  Per cube b the candidates are the cards of [0, C) NOT listed in mask row b;
+ * for every entry p in [target_ptr[b], target_ptr[b+1]), out_rank[p] is the 0-based position of card target_idx[p]
+ * among them in the descending order of cc_topn_masked_f32(descending = 1) / cc_topn_masked_sigmoid_f32: larger
+ * score first, ties -> larger index first, with apply_sigmoid != 0 the float32 sigmoid of the logits.  So a target of
+ * rank r < n is the one those selects return at slot r.  Targets are candidates too (a hidden card ranks behind the
+ * other hidden cards that beat it); a target listed in the mask or outside [0, C) gets -1; duplicate entries get the
+ * same rank.  Any number of targets per row.  NaN scores are outside the contract.  One CTA per cube: the row is read
+ * once per 1024 targets.  out_rank: int32 [target_ptr[batch]]. */
+int cc_rank_targets_f32(const float* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* mask_ptr,
+                        const int32_t* mask_idx, const int64_t* target_ptr, const int32_t* target_idx, int apply_sigmoid,
+                        int32_t* out_rank, void* stream);
 /* Card similarity (src/scripts/similarity.py:25-29): out[r] = -cos(emb[r], emb[query]) with Keras' l2_normalize
  * (epsilon 1e-12), emb float32 [rows][ld >= dim]; rank ascending with cc_topn_masked_f32. */
 int cc_cosine_neg_f32(const float* emb, int64_t ld, int32_t rows, int32_t dim, int32_t query, float* out, void* stream);
