@@ -52,6 +52,7 @@ SIGNATURES = {
     "cc_topn_rowselect_profile": (I, [P, I64, I32, I32, P, P, I32, I, P, P, P, P, P]),
     "cc_cuts_gather_f32": (I, [P, I64, I32, I32, P, P, I, P, P]),
     "cc_rank_targets_f32": (I, [P, I64, I32, I32, P, P, P, P, I, P, P]),
+    "cc_rank_targets_f64": (I, [P, I64, I32, I32, P, P, P, P, P, P]),
     "cc_cosine_neg_f32": (I, [P, I64, I32, I32, I32, P, P]),
     "cc_topn_masked_f64": (I, [P, I64, I32, I32, P, P, I, I, I32, P, I64, P, P, P, P]),
     # (3) noise

@@ -106,6 +106,11 @@ __device__ __forceinline__ float4 ld_nc_f4(const void* p) {
                : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
   return r;
 }
+__device__ __forceinline__ double2 ld_nc_d2(const void* p) {
+  double2 r;
+  asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0,%1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p));
+  return r;
+}
 // ---- the recommender's total order on (score, index): every select and the target-rank kernel ----------
 template <typename T> struct KeyOf;
 template <> struct KeyOf<float> {
@@ -164,6 +169,13 @@ __device__ __forceinline__ float rs_raw_bound(unsigned long long thr, int descen
   if (pp >= 1.f) return INFINITY;
   const float l = logf(pp / (1.f - pp));
   return l + rs_logit_slack(l, 1.f - pp);
+}
+// the float64 counterpart (no sigmoid): the threshold key's own double, decoded from its 64-bit score word
+__device__ __forceinline__ double rs_raw_bound_f64(unsigned __int128 thr, int descending) {
+  if (thr == 0) return descending ? -INFINITY : INFINITY;
+  unsigned long long u = (unsigned long long)(thr >> 32);
+  if (!descending) u = ~u;
+  return __longlong_as_double((long long)((u & 0x8000000000000000ull) ? (u ^ 0x8000000000000000ull) : ~u));
 }
 #endif
 

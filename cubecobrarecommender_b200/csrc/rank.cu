@@ -13,11 +13,25 @@ namespace cc {
 // j >= 1) and counted at cnt[j].  Target i (sorted) is beaten by exactly the elements with j > i: rank[i] =
 // sum_{j > i} cnt[j], one block scan.  Equal target keys (duplicate entries) share the first slot's rank: no element
 // has its j strictly between them.  A row with more than RT_CHUNK targets takes one sweep per chunk of them.
+// T = float (64-bit keys, optional fused sigmoid) or double (96-bit keys in an unsigned __int128, no sigmoid; ld == 0
+// is one score row shared by every cube).
 constexpr int RT_THREADS = 512;
 constexpr int RT_CHUNK = 2 * RT_THREADS;              // target keys per sweep (the scan gives each thread two of them)
-constexpr unsigned long long RT_NONE = ~0ull;         // not a candidate; no real key reaches it (its score word is a NaN)
 
-__device__ __forceinline__ int rt_count_below(const unsigned long long* keys, int m, unsigned long long k) {
+// not a candidate: all ones; no real key reaches it (its score word is a NaN)
+template <typename K> __device__ __forceinline__ K rt_none() { return ~K(0); }
+
+template <bool SIGMOID> __device__ __forceinline__ float rt_score(float x) { return SIGMOID ? sigmoid_f32(x) : x; }
+template <bool SIGMOID> __device__ __forceinline__ double rt_score(double x) { return x; }
+template <bool SIGMOID> __device__ __forceinline__ float rt_bound(unsigned long long thr) {
+  return rs_raw_bound<SIGMOID>(thr, 1);
+}
+template <bool SIGMOID> __device__ __forceinline__ double rt_bound(unsigned __int128 thr) {
+  return rs_raw_bound_f64(thr, 1);
+}
+
+template <typename K>
+__device__ __forceinline__ int rt_count_below(const K* keys, int m, K k) {
   int lo = 0, hi = m;                                  // #{i < m : keys[i] < k}, keys ascending
   while (lo < hi) {
     const int mid = (lo + hi) >> 1;
@@ -26,22 +40,25 @@ __device__ __forceinline__ int rt_count_below(const unsigned long long* keys, in
   return lo;
 }
 
-template <bool SIGMOID>
+template <typename T, bool SIGMOID>
 __global__ void __launch_bounds__(RT_THREADS, 2)
-rank_targets_kernel(const float* __restrict__ scores, int64_t ld, int32_t num_cards,
+rank_targets_kernel(const T* __restrict__ scores, int64_t ld, int32_t num_cards,
                     const int64_t* __restrict__ mask_ptr, const int32_t* __restrict__ mask_idx,
                     const int64_t* __restrict__ target_ptr, const int32_t* __restrict__ target_idx,
                     int32_t* __restrict__ out_rank) {
+  static_assert(!SIGMOID || sizeof(T) == 4, "the fused sigmoid ranks float32 logits");
+  using K = typename KeyOf<T>::K;
+  const K RT_NONE = rt_none<K>();
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  unsigned long long* keys = reinterpret_cast<unsigned long long*>(smem_raw);     // RT_CHUNK, sorted ascending
+  K* keys = reinterpret_cast<K*>(smem_raw);                                       // RT_CHUNK, sorted ascending
   int* cnt = reinterpret_cast<int*>(keys + RT_CHUNK);                             // RT_CHUNK + 1 counters, then ranks
   uint32_t* mask = reinterpret_cast<uint32_t*>(cnt + RT_CHUNK + 1);               // ceil(C/32) words
   __shared__ int s_warp[RT_THREADS / 32];
   __shared__ int s_m;
-  __shared__ float s_zb;
+  __shared__ T s_zb;
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   const int cube = blockIdx.x;
-  const float* sc = scores + int64_t(cube) * ld;
+  const T* sc = scores + int64_t(cube) * ld;
   const int words = (num_cards + 31) >> 5;
   for (int w = tid; w < words; w += RT_THREADS) mask[w] = 0u;
   __syncthreads();
@@ -50,18 +67,19 @@ rank_targets_kernel(const float* __restrict__ scores, int64_t ld, int32_t num_ca
     if (c >= 0 && c < num_cards) atomicOr(&mask[c >> 5], 1u << (c & 31));
   }
   __syncthreads();
-  auto target_key = [&](int32_t t) -> unsigned long long {
+  auto target_key = [&](int32_t t) -> K {
     if (t < 0 || t >= num_cards || ((mask[t >> 5] >> (t & 31)) & 1u)) return RT_NONE;
-    const float x = sc[t];
-    return make_key<float>(SIGMOID ? sigmoid_f32(x) : x, (uint32_t)t, 1);
+    const T x = sc[t];
+    return make_key<T>(rt_score<SIGMOID>(x), (uint32_t)t, 1);
   };
-  auto count = [&](float x, int e, float zb) {         // one candidate element against the chunk's target keys
+  auto count = [&](T x, int e, T zb) {                 // one candidate element against the chunk's target keys
     if (!(x >= zb) || ((mask[e >> 5] >> (e & 31)) & 1u)) return;
-    const unsigned long long k = make_key<float>(SIGMOID ? sigmoid_f32(x) : x, (uint32_t)e, 1);
+    const K k = make_key<T>(rt_score<SIGMOID>(x), (uint32_t)e, 1);
     const int m = s_m;
     if (k > keys[0]) atomicAdd(&cnt[rt_count_below(keys, m, k)], 1);
   };
-  const bool vec = (ld & 3) == 0 && (reinterpret_cast<uintptr_t>(scores) & 15) == 0;
+  // 16-byte rows: float with ld % 4 == 0, double with ld % 2 == 0 (ld == 0 included), on a 16-byte aligned base
+  const bool vec = (ld & (16 / sizeof(T) - 1)) == 0 && (reinterpret_cast<uintptr_t>(scores) & 15) == 0;
   const int64_t tb = target_ptr[cube], te = target_ptr[cube + 1];
 
   for (int64_t c0 = tb; c0 < te; c0 += RT_CHUNK) {
@@ -76,7 +94,7 @@ rank_targets_kernel(const float* __restrict__ scores, int64_t ld, int32_t num_ca
         for (int i = tid; i < n_pad; i += RT_THREADS) {
           const int ixj = i ^ j;
           if (ixj > i) {
-            const unsigned long long a = keys[i], b = keys[ixj];
+            const K a = keys[i], b = keys[ixj];
             if (((i & k) == 0) ? (a > b) : (a < b)) { keys[i] = b; keys[ixj] = a; }
           }
         }
@@ -87,12 +105,36 @@ rank_targets_kernel(const float* __restrict__ scores, int64_t ld, int32_t num_ca
     if (tid == 0 && keys[0] == RT_NONE) s_m = 0;
     for (int i = tid; i < n_pad; i += RT_THREADS)
       if (keys[i] != RT_NONE && (i + 1 == n_pad || keys[i + 1] == RT_NONE)) s_m = i + 1;
-    if (tid == 0 && keys[0] != RT_NONE) s_zb = rs_raw_bound<SIGMOID>(keys[0], 1);
+    if (tid == 0 && keys[0] != RT_NONE) s_zb = rt_bound<SIGMOID>(keys[0]);
     __syncthreads();
     const int m = s_m;
     if (m > 0) {
-      const float zb = s_zb;
-      if (vec) {
+      const T zb = s_zb;
+      if constexpr (sizeof(T) == 8) {
+        if (vec) {
+          // 16-byte loads of whole pairs, two in flight per thread; an odd row's last score is read alone (with
+          // ld == 0 the row may end right there)
+          const int c2 = num_cards >> 1;
+          for (int v = tid; v < c2; v += 2 * RT_THREADS) {
+            const int v1 = v + RT_THREADS;
+            const double2 q0 = ld_nc_d2(sc + 2 * v);
+            const double2 q1 = v1 < c2 ? ld_nc_d2(sc + 2 * v1) : make_double2(-INFINITY, -INFINITY);
+            const double2 qs[2] = {q0, q1};
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+              const double2 q = qs[u];
+              const int e0 = 2 * (u ? v1 : v);
+              // the sentinel pair past the row is skipped by index: with zb = -inf it would pass the value test
+              if ((u && v1 >= c2) || !(fmax(q.x, q.y) >= zb)) continue;
+              count(q.x, e0, zb);
+              count(q.y, e0 + 1, zb);
+            }
+          }
+          if ((num_cards & 1) && tid == 0) count(sc[num_cards - 1], num_cards - 1, zb);
+        } else {
+          for (int e = tid; e < num_cards; e += RT_THREADS) count(sc[e], e, zb);
+        }
+      } else if (vec) {
         // 16-byte loads, two in flight per thread; the float4 past the row's end stays inside ld (ld % 4 == 0)
         const int c4 = (num_cards + 3) >> 2;
         for (int v = tid; v < c4; v += 2 * RT_THREADS) {
@@ -144,7 +186,7 @@ rank_targets_kernel(const float* __restrict__ scores, int64_t ld, int32_t num_ca
     }
     __syncthreads();
     for (int i = tid; i < nt; i += RT_THREADS) {
-      const unsigned long long k = target_key(target_idx[c0 + i]);
+      const K k = target_key(target_idx[c0 + i]);
       out_rank[c0 + i] = k == RT_NONE ? -1 : cnt[rt_count_below(keys, m, k)];
     }
     __syncthreads();                                   // keys / cnt are refilled by the next chunk
@@ -170,15 +212,38 @@ int cc_rank_targets_f32(const float* scores, int64_t ld, int32_t num_cards, int3
   cudaStream_t st = as_stream(stream);
   if (apply_sigmoid) {
     if (smem > 48 * 1024)
-      CC_CHECK_CUDA(cudaFuncSetAttribute(rank_targets_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    rank_targets_kernel<true><<<batch, RT_THREADS, smem, st>>>(scores, ld, num_cards, mask_ptr, mask_idx, target_ptr,
-                                                               target_idx, out_rank);
+      CC_CHECK_CUDA(cudaFuncSetAttribute(rank_targets_kernel<float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem));
+    rank_targets_kernel<float, true><<<batch, RT_THREADS, smem, st>>>(scores, ld, num_cards, mask_ptr, mask_idx,
+                                                                      target_ptr, target_idx, out_rank);
   } else {
     if (smem > 48 * 1024)
-      CC_CHECK_CUDA(cudaFuncSetAttribute(rank_targets_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    rank_targets_kernel<false><<<batch, RT_THREADS, smem, st>>>(scores, ld, num_cards, mask_ptr, mask_idx, target_ptr,
-                                                                target_idx, out_rank);
+      CC_CHECK_CUDA(cudaFuncSetAttribute(rank_targets_kernel<float, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)smem));
+    rank_targets_kernel<float, false><<<batch, RT_THREADS, smem, st>>>(scores, ld, num_cards, mask_ptr, mask_idx,
+                                                                       target_ptr, target_idx, out_rank);
   }
+  CC_CHECK_LAUNCH();
+  return CC_OK;
+}
+
+int cc_rank_targets_f64(const double* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* mask_ptr,
+                        const int32_t* mask_idx, const int64_t* target_ptr, const int32_t* target_idx,
+                        int32_t* out_rank, void* stream) {
+  CC_NVTX("cc_rank_targets_f64");
+  CC_REQUIRE(scores && mask_ptr && mask_idx && target_ptr && target_idx && out_rank,
+             "cc_rank_targets_f64: null pointer");
+  CC_REQUIRE(num_cards >= 1 && batch >= 0 && (ld == 0 || ld >= num_cards),
+             "cc_rank_targets_f64: bad sizes (C=%d, batch=%d, ld=%lld)", num_cards, batch, (long long)ld);
+  if (batch == 0) return CC_OK;
+  const size_t smem = size_t(RT_CHUNK) * 16 + size_t(RT_CHUNK + 1) * 4 + size_t((num_cards + 31) / 32) * 4;
+  CC_REQUIRE(smem <= 200 * 1024, "cc_rank_targets_f64: C=%d needs %zu bytes of shared memory", num_cards, smem);
+  cudaStream_t st = as_stream(stream);
+  if (smem > 48 * 1024)
+    CC_CHECK_CUDA(cudaFuncSetAttribute(rank_targets_kernel<double, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
+  rank_targets_kernel<double, false><<<batch, RT_THREADS, smem, st>>>(scores, ld, num_cards, mask_ptr, mask_idx,
+                                                                      target_ptr, target_idx, out_rank);
   CC_CHECK_LAUNCH();
   return CC_OK;
 }

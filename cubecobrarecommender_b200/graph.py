@@ -5,6 +5,9 @@ Mirrors, on CSR cubes resident in HBM:
   * ``y_mtx`` / ``neg_sampler``         reference ``src/ml/train.py:69-71``, ``src/ml/generator.py:30``
   * ``simple_recs`` / ``simple_cuts``   reference ``src/scripts/recommend.py:7-18``, ``cut_cards.py:7-18``
 
+plus the leave-k-out ranks of the graph recommender and of a popularity ranking (the baselines the autoencoder's
+ranking metrics are read against, ``train.ranking_baselines``).
+
 Multi-GPU: cubes are sharded across ranks; each rank counts its own shard into a private
 int32 ``(C, C)`` and one NCCL ``all_reduce(SUM)`` combines them (exact, order independent).
 """
@@ -223,27 +226,44 @@ def topn_masked(scores: torch.Tensor, mask_ptr: torch.Tensor, mask_idx: torch.Te
 
 def rank_targets(scores: torch.Tensor, mask_ptr: torch.Tensor, mask_idx: torch.Tensor, target_ptr: torch.Tensor,
                  target_idx: torch.Tensor, *, sigmoid=False, out=None) -> torch.Tensor:
-    """int32 rank of every target entry (cc_rank_targets_f32): the 0-based slot at which the descending
+    """int32 rank of every target entry (cc_rank_targets_f32 / _f64): the 0-based slot at which the descending
     :func:`topn_masked` select over the cards not listed in the mask row would return it, or -1 for a target that is
-    masked or out of range.  ``scores`` float32 (batch, >= C) with unit column stride, C = ``scores.shape[1]``;
-    ``sigmoid=True``: ``scores`` are logits, ranked by their float32 sigmoid.  ``out``: int32, one entry per
-    ``target_idx`` entry (default: allocated)."""
-    if scores.dtype != torch.float32 or scores.dim() != 2 or scores.stride(1) != 1:
-        raise TypeError("scores must be a float32 (batch, C) tensor with unit column stride")
+    masked or out of range.  ``scores`` float32 or float64 (batch, >= C) with unit column stride, C =
+    ``scores.shape[1]``; float64 rows may also have stride 0 (``row.expand(batch, C)``: one row ranked for every cube).
+    ``sigmoid=True`` (float32 only): ``scores`` are logits, ranked by their float32 sigmoid.  ``out``: int32, one entry
+    per ``target_idx`` entry (default: allocated)."""
+    if scores.dtype not in (torch.float32, torch.float64) or scores.dim() != 2 or scores.stride(1) != 1:
+        raise TypeError("scores must be a float32 or float64 (batch, C) tensor with unit column stride")
     if out is None:
         out = torch.empty(target_idx.numel(), dtype=torch.int32, device=scores.device)
+    if scores.dtype == torch.float64:
+        if sigmoid:
+            raise TypeError("the fused sigmoid ranks float32 logits")
+        call("cc_rank_targets_f64", ptr(scores), scores.stride(0), int(scores.shape[1]), int(scores.shape[0]),
+             ptr(mask_ptr), ptr(mask_idx), ptr(target_ptr), ptr(target_idx), ptr(out), stream_ptr())
+        return out
     call("cc_rank_targets_f32", ptr(scores), scores.stride(0), int(scores.shape[1]), int(scores.shape[0]),
          ptr(mask_ptr), ptr(mask_idx), ptr(target_ptr), ptr(target_idx), int(sigmoid), ptr(out), stream_ptr())
     return out
 
 
-class GraphRecommender:
-    """M resident in HBM (float64); batched ``simple_recs`` / ``simple_cuts``."""
+def _check_holdout_pair(visible: CubeCSR, hidden: CubeCSR, num_cards: int):
+    if hidden.num_cubes != visible.num_cubes or hidden.num_cards != visible.num_cards:
+        raise ValueError("visible and hidden must hold the same cubes over the same cards")
+    if visible.num_cards != num_cards:
+        raise ValueError(f"the cubes span {visible.num_cards} cards, the recommender {num_cards}")
 
-    def __init__(self, m64: torch.Tensor):
+
+class GraphRecommender:
+    """M resident in HBM (float64); batched ``simple_recs`` / ``simple_cuts``.  ``budget_bytes``: device memory one
+    chunk of :meth:`target_ranks_device` may take for its leaf partials and score rows."""
+
+    def __init__(self, m64: torch.Tensor, budget_bytes: int = 1 << 30):
         assert m64.dtype == torch.float64 and m64.dim() == 2
         self.m = m64.contiguous()
         self.num_cards = m64.shape[0]
+        self.device = self.m.device
+        self.budget_bytes = int(budget_bytes)
 
     def scores(self, csr: CubeCSR, zero_diag=False) -> torch.Tensor:
         lib = _lib.load()
@@ -274,3 +294,94 @@ class GraphRecommender:
         """``n`` lowest-scored in-cube cards per cube, ascending (cut_cards.py:7-18)."""
         scores, row_ptr, rows = self.scores(csr, zero_diag=True)
         return topn_masked(scores, row_ptr, rows, n, only_listed=True, descending=False)
+
+    def target_ranks_device(self, visible: CubeCSR, hidden: CubeCSR) -> torch.Tensor:
+        """Leave-k-out ranks, int32 aligned with ``hidden.indices``, on the device: each hidden card of cube b gets the
+        0-based slot at which :meth:`recs` (and so ``simple_recs``) would list it for the cube's ``visible`` cards, or
+        -1 if it is also visible.  The cubes are scored in chunks (the float64 sums of :meth:`scores`, NumPy's pairwise
+        order) whose leaf partials and score rows fit ``budget_bytes``, then ranked by cc_rank_targets_f64.  Chunk
+        i+1's plan is built on the host and its rows are uploaded on a copy stream while chunk i computes; nothing
+        synchronises with the host."""
+        _check_holdout_pair(visible, hidden, self.num_cards)
+        lib = _lib.load()
+        dev, c, k = self.device, self.num_cards, visible.num_cubes
+        vp = np.ascontiguousarray(visible.indptr, dtype=np.int64)
+        vi = np.ascontiguousarray(visible.indices, dtype=np.int32)
+        hp = np.ascontiguousarray(hidden.indptr, dtype=np.int64)
+        hi_ = np.ascontiguousarray(hidden.indices, dtype=np.int32)
+        ranks = torch.empty(max(int(hp[-1]), 1), dtype=torch.int32, device=dev)
+        if k == 0:
+            return ranks[:0]
+        sizes = np.diff(vp)
+        uniq, inv = np.unique(sizes, return_inverse=True)
+        leaves = np.array([lib.cc_pairwise_leaf_count(int(n)) if n > 0 else 0 for n in uniq], dtype=np.int64)[inv]
+        # a cube costs its leaf partials plus its score row; every chunk takes at least one cube
+        cum = np.concatenate([[0], np.cumsum((leaves + 1) * c * 8)])
+        bounds = [0]
+        while bounds[-1] < k:
+            lo = bounds[-1]
+            bounds.append(max(lo + 1, int(np.searchsorted(cum, cum[lo] + self.budget_bytes, side="right")) - 1))
+        spans = list(zip(bounds[:-1], bounds[1:]))
+        max_leaves = max(int(leaves[lo:hi].sum()) for lo, hi in spans)
+        max_cubes = max(hi - lo for lo, hi in spans)
+        partial = torch.empty((max(max_leaves, 1), c), dtype=torch.float64, device=dev)
+        scores = torch.empty((max_cubes, c), dtype=torch.float64, device=dev)
+        compute = torch.cuda.current_stream(dev)
+        copier = self._copy_stream = getattr(self, "_copy_stream", None) or torch.cuda.Stream(device=dev)
+
+        def upload(lo, hi):
+            nl = int(leaves[lo:hi].sum())
+            row_ptr_h = vp[lo:hi + 1] - vp[lo]
+            plan_h = np.zeros((max(nl, 1), 4), dtype=np.int32)
+            leaf_ptr_h = np.zeros(hi - lo + 1, dtype=np.int32)
+            call("cc_pairwise_plan_host", ptr(row_ptr_h), hi - lo, ptr(plan_h), ptr(leaf_ptr_h))
+            arrays = (vi[vp[lo]:vp[hi]], row_ptr_h, plan_h, leaf_ptr_h, hi_[hp[lo]:hp[hi]], hp[lo:hi + 1] - hp[lo])
+            with torch.cuda.stream(copier):
+                parts = [torch.from_numpy(a if len(a) else np.zeros(1, a.dtype)).to(dev, non_blocking=True)
+                         for a in arrays]
+                ev = torch.cuda.Event()
+                ev.record(copier)
+            for t in parts:
+                t.record_stream(compute)           # allocated on the copy stream, consumed on the compute stream
+            return lo, hi, nl, parts, ev
+
+        nxt = upload(*spans[0])
+        for i in range(len(spans)):
+            lo, hi, nl, (rows, row_ptr, plan, leaf_ptr, t_idx, t_ptr), ev = nxt
+            nxt = upload(*spans[i + 1]) if i + 1 < len(spans) else None       # overlaps this chunk's kernels
+            compute.wait_event(ev)
+            sc = scores[:hi - lo]
+            call("cc_score_gather_f64", ptr(self.m), self.m.stride(0), c, ptr(rows), ptr(row_ptr), hi - lo, ptr(plan),
+                 ptr(leaf_ptr), nl, 0, ptr(partial), ptr(sc), sc.stride(0), stream_ptr())
+            if hp[hi] > hp[lo]:
+                rank_targets(sc, row_ptr, rows, t_ptr, t_idx, out=ranks[int(hp[lo]):int(hp[hi])])
+        return ranks[:int(hp[-1])]
+
+
+class PopularityRecommender:
+    """The popularity floor: every cube gets the same ranking, the cards listed by the most training cubes first (ties
+    to the larger index, the order of every select), minus the cube's own cards.  ``scores`` is one float64 row, the
+    number of cubes of ``csr`` that list each card (rows are sets)."""
+
+    def __init__(self, csr: CubeCSR, device="cuda"):
+        counts = np.bincount(np.asarray(csr.indices, dtype=np.int64), minlength=csr.num_cards)
+        self.num_cards = csr.num_cards
+        self.device = torch.device(device)
+        self.scores = torch.from_numpy(counts.astype(np.float64)).to(self.device)
+
+    def target_ranks_device(self, visible: CubeCSR, hidden: CubeCSR) -> torch.Tensor:
+        """Leave-k-out ranks, int32 aligned with ``hidden.indices``, on the device: each hidden card's 0-based slot in
+        the popularity list without the cube's ``visible`` cards, or -1 if it is also visible.  One cc_rank_targets_f64
+        launch over every cube, all reading the one score row (row stride 0)."""
+        _check_holdout_pair(visible, hidden, self.num_cards)
+        k = visible.num_cubes
+        hp = np.ascontiguousarray(hidden.indptr, dtype=np.int64)
+        ranks = torch.empty(max(int(hp[-1]), 1), dtype=torch.int32, device=self.device)
+        if k == 0 or hp[-1] == 0:
+            return ranks[:int(hp[-1])]
+        mp, mi = upload_csr(visible, self.device)
+        tp, ti = upload_csr(hidden, self.device)
+        if mi.numel() == 0:                    # no visible card anywhere: a valid (never read) mask pointer
+            mi = mi.new_zeros(1)
+        rank_targets(self.scores.expand(k, self.num_cards), mp, mi, tp, ti, out=ranks)
+        return ranks

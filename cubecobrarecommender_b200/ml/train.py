@@ -1,7 +1,7 @@
 """Drop-in for reference ``src/ml/train.py``.
 
     python -m cubecobrarecommender_b200.ml.train epochs batch_size name reg noise [seed] [--validation-split F]
-                                                 [--rank-at K1,K2,...]
+                                                 [--rank-at K1,K2,...] [--rank-baselines graph,popularity]
 
 Same positional arguments (reference train.py:28-38), same inputs (``data/maps/nameToId.json``,
 ``data/cube/*.json``, ``output/full_adj_mtx.npy``), same M-hat construction (train.py:69-71), loss and
@@ -84,7 +84,10 @@ def evaluate_recommendations(model, generator, *, at=(10, 50), holdout=0.2, grou
     """Leave-k-out ranking quality of the recommendations over every cube of ``generator``: each cube of s >= 2 cards
     hides ``min(s - 1, max(1, floor(holdout * s + 0.5)))`` of them (``DataGenerator.holdout_split``: the same cards in
     every call), the model sees the rest, and every hidden card is ranked among all the cards the cube does not show,
-    in the order ``MLRecommender.recommend_device`` lists them.  Returns ``{"recall_at_k", "ndcg_at_k",
+    in the order ``MLRecommender.recommend_device`` lists them.  ``model``: a ``CC_Recommender`` (ranked through
+    ``MLRecommender``) or any recommender with ``target_ranks_device(visible, hidden)`` -- ``MLRecommender``,
+    ``graph.GraphRecommender``, ``graph.PopularityRecommender`` -- so the baselines are scored on the same hidden cards
+    by the same code (see ``ranking_baselines``).  Returns ``{"recall_at_k", "ndcg_at_k",
     "hit_rate_at_k"}`` for each k in ``at``, ``"mrr"``, ``"mpr"`` (mean percentile rank: 0.5 for a random ranking) --
     each a mean over the evaluated cubes, see ``ranking.ranking_sums`` -- plus ``"cubes"`` (evaluated) and ``"skipped"``
     (fewer than two cards).  Under ``torchrun`` each rank takes a contiguous shard of the cubes and one all_reduce adds
@@ -93,6 +96,7 @@ def evaluate_recommendations(model, generator, *, at=(10, 50), holdout=0.2, grou
     ones included."""
     import torch.distributed as dist
     from .inference import MLRecommender
+    from .model import CC_Recommender
     from .ranking import metric_names, ranking_sums
     at = tuple(int(k) for k in at)
     if not at or min(at) < 1:
@@ -104,8 +108,9 @@ def evaluate_recommendations(model, generator, *, at=(10, 50), holdout=0.2, grou
         raise ValueError("evaluate_recommendations: the generator holds no cubes")
     visible, hidden, _ = generator.holdout_split(holdout)
     vis, hid = visible.shard(rank, world), hidden.shard(rank, world)          # the cubes of shard_range(k, rank, world)
-    dev = model.device
-    ranks = MLRecommender(model).target_ranks_device(vis, hid)
+    rec = MLRecommender(model) if isinstance(model, CC_Recommender) else model
+    ranks = rec.target_ranks_device(vis, hid)
+    dev = ranks.device
     hp = torch.from_numpy(np.ascontiguousarray(hid.indptr, dtype=np.int64)).to(dev, non_blocking=True)
     n_cand = torch.from_numpy(generator.N_cards - np.diff(vis.indptr)).to(dev, non_blocking=True)
     sums = ranking_sums(ranks, hp, n_cand, at)
@@ -115,6 +120,36 @@ def evaluate_recommendations(model, generator, *, at=(10, 50), holdout=0.2, grou
     cubes = int(round(t[0]))
     out = {name: float(v / cubes) if cubes else float("nan") for name, v in zip(metric_names(at), t[1:])}
     out.update({"cubes": cubes, "skipped": k - cubes})
+    return out
+
+
+BASELINES = ("graph", "popularity")
+
+
+def ranking_baselines(train_generator, val_generator, *, names=BASELINES, at, holdout, group=None):
+    """``{name: evaluate_recommendations(...)}`` of simple recommenders on ``val_generator``'s cubes, the same hidden
+    cards and metrics as the autoencoder's ranking evaluation, to read its numbers against.  ``"graph"``: the
+    co-occurrence recommender (``simple_recs``, reference ``recommend.py:7-18``) with M built from the cubes of
+    ``train_generator`` only, so no held-out co-occurrence leaks into it (the autoencoder's M-hat, by contrast, is built
+    from every cube).  ``"popularity"``: the cards listed by the most training cubes, the same list for every cube.
+    Under ``torchrun`` every rank builds the whole graph (no all_reduce of the counts) and ranks its shard of the
+    validation cubes; the graph is freed before the function returns."""
+    from .. import graph as G
+    names = tuple(names)
+    unknown = [n for n in names if n not in BASELINES]
+    if unknown:
+        raise ValueError(f"unknown ranking baseline(s) {unknown}; choose from {list(BASELINES)}")
+    out = {}
+    for name in names:
+        if name == "graph":
+            g = G.build_graph(train_generator.csr, train_generator.device, allreduce=False, want_m64=True,
+                              want_mhat=False, want_neg=False)
+            rec = G.GraphRecommender(g.m64)
+            del g                                           # the int32 counts go now, M with the recommender below
+        else:
+            rec = G.PopularityRecommender(train_generator.csr, train_generator.device)
+        out[name] = evaluate_recommendations(rec, val_generator, at=at, holdout=holdout, group=group)
+        del rec
     return out
 
 
@@ -208,7 +243,7 @@ def parse_args(argv):
     resume = "--resume" in args
     if resume:
         args.remove("--resume")
-    flags = {"--save-every": None, "--validation-split": 0.0, "--rank-at": None}
+    flags = {"--save-every": None, "--validation-split": 0.0, "--rank-at": None, "--rank-baselines": None}
     for flag in flags:
         if flag in args:
             i = args.index(flag)
@@ -218,7 +253,7 @@ def parse_args(argv):
             del args[i:i + 2]
     if len(args) < 5:
         raise SystemExit("usage: train.py epochs batch_size name reg noise [seed] [--save-every N] [--resume] "
-                         "[--validation-split F] [--rank-at K1,K2,...]")
+                         "[--validation-split F] [--rank-at K1,K2,...] [--rank-baselines graph,popularity]")
     split = float(flags["--validation-split"])
     if not 0.0 <= split < 1.0:
         raise SystemExit(f"--validation-split must lie in [0, 1), got {split}")
@@ -232,10 +267,19 @@ def parse_args(argv):
             raise SystemExit(f"--rank-at values must be >= 1, got {flags['--rank-at']}")
         if split == 0.0:
             raise SystemExit("--rank-at ranks the held-out cubes: it needs --validation-split F")
+    baselines = None
+    if flags["--rank-baselines"] is not None:
+        baselines = tuple(v for v in flags["--rank-baselines"].split(",") if v)
+        unknown = [v for v in baselines if v not in BASELINES]
+        if not baselines or unknown:
+            raise SystemExit(f"--rank-baselines takes a comma-separated list of {', '.join(BASELINES)}, "
+                             f"got {flags['--rank-baselines']!r}")
+        if rank_at is None:
+            raise SystemExit("--rank-baselines reports the metrics of --rank-at: it needs --rank-at K1,K2,...")
     return {"epochs": int(args[0]), "batch_size": int(args[1]), "name": args[2], "reg": float(args[3]),
             "noise": float(args[4]), "seed": int(args[5]) if len(args) == 6 else 0, "seed_given": len(args) == 6,
             "resume": resume, "save_every": int(flags["--save-every"]) if flags["--save-every"] is not None else None,
-            "validation_split": split, "rank_at": rank_at}
+            "validation_split": split, "rank_at": rank_at, "rank_baselines": baselines}
 
 
 def main(argv=None):
@@ -244,7 +288,9 @@ def main(argv=None):
     continues from the checkpoint found there (weights, Adam slots, step counter, completed epochs),
     ``--validation-split F`` holds the last fraction F of the cubes out of training and reports ``val_*`` losses and
     accuracies on them after every epoch, ``--rank-at 10,50`` adds the leave-k-out ranking metrics of those cubes
-    (``val_recall_at_10``, ``val_ndcg_at_10``, ``val_hit_rate_at_10``, ..., ``val_mrr``, ``val_mpr``)."""
+    (``val_recall_at_10``, ``val_ndcg_at_10``, ``val_hit_rate_at_10``, ..., ``val_mrr``, ``val_mpr``), and
+    ``--rank-baselines graph,popularity`` prints the same metrics of those baselines (``ranking_baselines``) on the
+    same cubes before the first epoch, one ``baseline <name> - recall_at_10: ...`` line each."""
     from ..non_ml import utils
     from .generator import DataGenerator
     from .model import CC_Recommender
@@ -280,6 +326,13 @@ def main(argv=None):
     else:
         autoencoder = CC_Recommender(num_cards, device="cuda", seed=seed, precision=precision)
     generator = DataGenerator(y_mtx, cubes, batch_size=batch_size, noise=noise, seed=seed)
+    if opts["rank_baselines"]:
+        from .ranking import metric_names
+        train_gen, val_gen = generator.split(opts["validation_split"])          # the halves fit's split makes
+        for bname, logs in ranking_baselines(train_gen, val_gen, names=opts["rank_baselines"],
+                                             at=opts["rank_at"], holdout=0.2).items():   # fit's ranking_holdout
+            print(f"baseline {bname}" + "".join(f" - {key}: {logs[key]:.4f}" for key in metric_names(opts["rank_at"])))
+        del train_gen, val_gen
     fit(autoencoder, generator, epochs, reg, initial_epoch=initial_epoch, checkpoint_dir=dest, save_every=save_every,
         validation_split=opts["validation_split"], ranking_at=opts["rank_at"])
     if not dist.is_initialized() or dist.get_rank() == 0:

@@ -153,6 +153,14 @@ int cc_cuts_gather_f32(const float* scores, int64_t ld, int32_t num_cards, int32
 int cc_rank_targets_f32(const float* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* mask_ptr,
                         const int32_t* mask_idx, const int64_t* target_ptr, const int32_t* target_idx, int apply_sigmoid,
                         int32_t* out_rank, void* stream);
+/* The same ranks for float64 scores, in the order of cc_topn_masked_f64(descending = 1): larger score first, ties ->
+ * larger index first (so a target of rank r < n is the one that select returns at slot r).  No sigmoid.  ld == 0 means
+ * one score row shared by every cube (e.g. a popularity ranking); otherwise ld >= C.  Masked, out-of-range and
+ * duplicate targets as in cc_rank_targets_f32; NaN scores are outside the contract.  out_rank: int32
+ * [target_ptr[batch]]. */
+int cc_rank_targets_f64(const double* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* mask_ptr,
+                        const int32_t* mask_idx, const int64_t* target_ptr, const int32_t* target_idx,
+                        int32_t* out_rank, void* stream);
 /* Card similarity (src/scripts/similarity.py:25-29): out[r] = -cos(emb[r], emb[query]) with Keras' l2_normalize
  * (epsilon 1e-12), emb float32 [rows][ld >= dim]; rank ascending with cc_topn_masked_f32. */
 int cc_cosine_neg_f32(const float* emb, int64_t ld, int32_t rows, int32_t dim, int32_t query, float* out, void* stream);

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Per-kernel comparison of two builds of one CUDA source: SASS instruction text, opcode histogram and the
 `-Xptxas -v` register / spill lines of every kernel the old object has.  A kernel that gained a defaulted template
-argument (e.g. `softmax_kl_regs_kernel<F, T, I>` -> `<F, T, I, true>`) is matched to its old name.
+argument (e.g. `softmax_kl_regs_kernel<F, T, I>` -> `<F, T, I, true>`), or a leading `float` score-type argument
+(e.g. `rank_targets_kernel<true>` -> `<float, true>`), is matched to its old name.
 
     nvcc ... -Xptxas -v -c src.cu -o old.o 2> old.ptxas      (parent commit)
     nvcc ... -Xptxas -v -c src.cu -o new.o 2> new.ptxas      (this change)
@@ -49,6 +50,7 @@ for n in b:
     d = demangle(n)
     new_by_old[d] = n
     new_by_old.setdefault(re.sub(r", true>$", ">", d), n)
+    new_by_old.setdefault(re.sub(r"<float, ", "<", d), n)
 same = 0
 for n in sorted(a, key=demangle):
     d = demangle(n)
