@@ -47,6 +47,17 @@ def _to_bf16(src, dst):
     call("cc_convert_f32_bf16", ptr(src), src.stride(0), ptr(dst), dst.stride(0), src.shape[0], src.shape[1], stream_ptr())
 
 
+def categorical_hits(z, rows, num_cards, target_rows, target_argmax, row_hit):
+    """Keras' categorical_accuracy of the softmax tower for row shapes the persistent softmax-KL kernel does not take
+    (num_cards % 4 != 0 or more than 25 600 cards): ``row_hit[i] = 1`` where the first maximal logit of ``z[i, :num_cards]``
+    sits in column ``target_argmax[target_rows[i]]``, for i < ``rows``.  The logits' argmax is cc_kl_target_argmax, the
+    same first-maximum rule the persistent kernels count with.  Device work only, no host sync; ``z`` must still hold
+    the logits (call it before the softmax-KL kernel turns them into dlogits)."""
+    am = torch.empty(rows, dtype=torch.int32, device=z.device)
+    call("cc_kl_target_argmax", ptr(z), z.stride(0), rows, num_cards, ptr(am), stream_ptr())
+    row_hit[:rows].copy_(am == target_argmax[target_rows[:rows].long()])
+
+
 def full_identity_shard(num_cards: int, rank: int = 0, world: int = 1):
     """Rows of I (cards) that rank ``rank`` of ``world`` regularises in full-I mode: an exact partition of
     ``[0, C)`` (shard sizes differ by at most one; each rank builds its engine with its own shard size)."""
@@ -513,15 +524,17 @@ class DAEEngine:
                              self.dz2_16.stride(0), ptr(self.kl_table()), ptr(self.kl_argmax()) if want_hit else None,
                              ptr(row_hit) if want_hit else None, st)
                     else:
-                        if want_hit and not reg_dbias_fused:
-                            raise RuntimeError("metrics need the persistent softmax-KL kernel (num_cards % 4 == 0, C <= 25600)")
+                        hit_in_kernel = want_hit and reg_dbias_fused
+                        if want_hit and not reg_dbias_fused:      # only the persistent kernels count hits
+                            categorical_hits(self.z2, Rm, self.C, rr, self.kl_argmax(), row_hit)
+                            n_launch += 1
                         call("cc_softmax_kl_fwd_bwd_metrics", ptr(self.z2), self.z2.stride(0), ptr(self.mhat), self.mhat.stride(0),
                              ptr(rr), Rm, self.C, self.cpad, self.reg / float(self.global_R), ptr(self.z2),
                              self.z2.stride(0), ptr(row_kl), int(tc),
                              ptr(dbias) if reg_dbias_fused else None, None, 0,
                              ptr(self.kl_table()) if reg_dbias_fused else None,
-                             ptr(self.kl_argmax()) if want_hit else None,
-                             ptr(row_hit) if want_hit else None, st)
+                             ptr(self.kl_argmax()) if hit_in_kernel else None,
+                             ptr(row_hit) if hit_in_kernel else None, st)
             n_launch += 1
         if ev:
             sums[0] += (eb["part"] if tc else eb["bce"][:Bm]).sum()
