@@ -5,8 +5,8 @@ Mirrors, on CSR cubes resident in HBM:
   * ``y_mtx`` / ``neg_sampler``         reference ``src/ml/train.py:69-71``, ``src/ml/generator.py:30``
   * ``simple_recs`` / ``simple_cuts``   reference ``src/scripts/recommend.py:7-18``, ``cut_cards.py:7-18``
 
-plus the leave-k-out ranks of the graph recommender and of a popularity ranking (the baselines the autoencoder's
-ranking metrics are read against, ``train.ranking_baselines``).
+plus the leave-k-out and cut ranks of the graph recommender and of a popularity ranking (the baselines the
+autoencoder's ranking metrics are read against, ``train.ranking_baselines``).
 
 Multi-GPU: cubes are sharded across ranks; each rank counts its own shard into a private
 int32 ``(C, C)`` and one NCCL ``all_reduce(SUM)`` combines them (exact, order independent).
@@ -247,9 +247,30 @@ def rank_targets(scores: torch.Tensor, mask_ptr: torch.Tensor, mask_idx: torch.T
     return out
 
 
-def _check_holdout_pair(visible: CubeCSR, hidden: CubeCSR, num_cards: int):
+def rank_cuts(scores: torch.Tensor, list_ptr: torch.Tensor, list_idx: torch.Tensor, target_ptr: torch.Tensor,
+              target_idx: torch.Tensor, *, sigmoid=False, out=None) -> torch.Tensor:
+    """int32 cut rank of every target entry (cc_rank_cuts_f32 / _f64): the 0-based slot at which the ascending
+    :func:`topn_masked` select over the cards listed in the row (``only_listed=True, descending=False``, the cut list)
+    would return it, or -1 for a target that is not listed or out of range.  Scores, strides, ``sigmoid`` and ``out`` as
+    in :func:`rank_targets`."""
+    if scores.dtype not in (torch.float32, torch.float64) or scores.dim() != 2 or scores.stride(1) != 1:
+        raise TypeError("scores must be a float32 or float64 (batch, C) tensor with unit column stride")
+    if out is None:
+        out = torch.empty(target_idx.numel(), dtype=torch.int32, device=scores.device)
+    if scores.dtype == torch.float64:
+        if sigmoid:
+            raise TypeError("the fused sigmoid ranks float32 logits")
+        call("cc_rank_cuts_f64", ptr(scores), scores.stride(0), int(scores.shape[1]), int(scores.shape[0]),
+             ptr(list_ptr), ptr(list_idx), ptr(target_ptr), ptr(target_idx), ptr(out), stream_ptr())
+        return out
+    call("cc_rank_cuts_f32", ptr(scores), scores.stride(0), int(scores.shape[1]), int(scores.shape[0]),
+         ptr(list_ptr), ptr(list_idx), ptr(target_ptr), ptr(target_idx), int(sigmoid), ptr(out), stream_ptr())
+    return out
+
+
+def _check_holdout_pair(visible: CubeCSR, hidden: CubeCSR, num_cards: int, names=("visible", "hidden")):
     if hidden.num_cubes != visible.num_cubes or hidden.num_cards != visible.num_cards:
-        raise ValueError("visible and hidden must hold the same cubes over the same cards")
+        raise ValueError(f"{names[0]} and {names[1]} must hold the same cubes over the same cards")
     if visible.num_cards != num_cards:
         raise ValueError(f"the cubes span {visible.num_cards} cards, the recommender {num_cards}")
 
@@ -303,12 +324,25 @@ class GraphRecommender:
         i+1's plan is built on the host and its rows are uploaded on a copy stream while chunk i computes; nothing
         synchronises with the host."""
         _check_holdout_pair(visible, hidden, self.num_cards)
+        return self._chunked_ranks(visible, hidden, 0, rank_targets)
+
+    def cut_ranks_device(self, corrupted: CubeCSR, intruders: CubeCSR) -> torch.Tensor:
+        """Cut ranks, int32 aligned with ``intruders.indices``, on the device: each intruder of cube b gets the 0-based
+        slot at which :meth:`cuts` (and so ``simple_cuts``) would list it among the cube's ``corrupted`` cards, or -1
+        if it is not one of them.  The chunks of :meth:`target_ranks_device`, scored with M's diagonal zeroed (the
+        scores of :meth:`cuts`) and ranked by cc_rank_cuts_f64; nothing synchronises with the host."""
+        _check_holdout_pair(corrupted, intruders, self.num_cards, ("corrupted", "intruders"))
+        return self._chunked_ranks(corrupted, intruders, 1, rank_cuts)
+
+    def _chunked_ranks(self, inputs: CubeCSR, targets: CubeCSR, zero_diag: int, rank) -> torch.Tensor:
+        """``rank(scores, row_ptr, rows, target_ptr, target_idx, out=...)`` of every chunk of cubes, the scores being
+        those of :meth:`scores` over the ``inputs`` rows: int32 ranks aligned with ``targets.indices``."""
         lib = _lib.load()
-        dev, c, k = self.device, self.num_cards, visible.num_cubes
-        vp = np.ascontiguousarray(visible.indptr, dtype=np.int64)
-        vi = np.ascontiguousarray(visible.indices, dtype=np.int32)
-        hp = np.ascontiguousarray(hidden.indptr, dtype=np.int64)
-        hi_ = np.ascontiguousarray(hidden.indices, dtype=np.int32)
+        dev, c, k = self.device, self.num_cards, inputs.num_cubes
+        vp = np.ascontiguousarray(inputs.indptr, dtype=np.int64)
+        vi = np.ascontiguousarray(inputs.indices, dtype=np.int32)
+        hp = np.ascontiguousarray(targets.indptr, dtype=np.int64)
+        hi_ = np.ascontiguousarray(targets.indices, dtype=np.int32)
         ranks = torch.empty(max(int(hp[-1]), 1), dtype=torch.int32, device=dev)
         if k == 0:
             return ranks[:0]
@@ -352,9 +386,9 @@ class GraphRecommender:
             compute.wait_event(ev)
             sc = scores[:hi - lo]
             call("cc_score_gather_f64", ptr(self.m), self.m.stride(0), c, ptr(rows), ptr(row_ptr), hi - lo, ptr(plan),
-                 ptr(leaf_ptr), nl, 0, ptr(partial), ptr(sc), sc.stride(0), stream_ptr())
+                 ptr(leaf_ptr), nl, zero_diag, ptr(partial), ptr(sc), sc.stride(0), stream_ptr())
             if hp[hi] > hp[lo]:
-                rank_targets(sc, row_ptr, rows, t_ptr, t_idx, out=ranks[int(hp[lo]):int(hp[hi])])
+                rank(sc, row_ptr, rows, t_ptr, t_idx, out=ranks[int(hp[lo]):int(hp[hi])])
         return ranks[:int(hp[-1])]
 
 
@@ -384,4 +418,21 @@ class PopularityRecommender:
         if mi.numel() == 0:                    # no visible card anywhere: a valid (never read) mask pointer
             mi = mi.new_zeros(1)
         rank_targets(self.scores.expand(k, self.num_cards), mp, mi, tp, ti, out=ranks)
+        return ranks
+
+    def cut_ranks_device(self, corrupted: CubeCSR, intruders: CubeCSR) -> torch.Tensor:
+        """Cut ranks, int32 aligned with ``intruders.indices``, on the device: each intruder's 0-based slot among the
+        cube's ``corrupted`` cards ordered least listed first (ties to the smaller index, the ascending select's
+        order), or -1 if it is not one of them.  One cc_rank_cuts_f64 launch over every cube (row stride 0)."""
+        _check_holdout_pair(corrupted, intruders, self.num_cards, ("corrupted", "intruders"))
+        k = corrupted.num_cubes
+        tp_h = np.ascontiguousarray(intruders.indptr, dtype=np.int64)
+        ranks = torch.empty(max(int(tp_h[-1]), 1), dtype=torch.int32, device=self.device)
+        if k == 0 or tp_h[-1] == 0:
+            return ranks[:int(tp_h[-1])]
+        cp, ci = upload_csr(corrupted, self.device)
+        tp, ti = upload_csr(intruders, self.device)
+        if ci.numel() == 0:                    # no listed card anywhere: a valid (never read) list pointer
+            ci = ci.new_zeros(1)
+        rank_cuts(self.scores.expand(k, self.num_cards), cp, ci, tp, ti, out=ranks)
         return ranks

@@ -61,6 +61,7 @@ class DataGenerator:
         self._step = torch.zeros(1, dtype=torch.int64, device=self.device)
         self._validation = None
         self._holdout = None
+        self._intruders = None
 
     def split(self, validation_split: float):
         """``(train, val)`` generators: Keras' ``validation_split`` -- the validation cubes are the last
@@ -84,6 +85,7 @@ class DataGenerator:
         g._step = torch.zeros(1, dtype=torch.int64, device=self.device)
         g._validation = None
         g._holdout = None
+        g._intruders = None
         g.reset_indices()
         return g
 
@@ -115,6 +117,20 @@ class DataGenerator:
             seed = (self.seed * 0x9E3779B97F4A7C15 + HOLDOUT_SEED_SALT) % (1 << 64)
             self._holdout[fraction] = holdout_split(self.csr, fraction, seed)
         return self._holdout[fraction]
+
+    def intruder_split(self, fraction: float):
+        """``(corrupted, intruders, evaluated)`` of ``ranking.intruder_split`` over this generator's cubes, with a seed
+        of its own (the generator seed mixed with ``ranking.INTRUDER_SEED_SALT``): computed once per fraction on the
+        host over the whole set (a donor may lie in any shard), so every epoch injects the same cards, and no random
+        stream of the generator is drawn from."""
+        from .ranking import INTRUDER_SEED_SALT, intruder_split
+        if self._intruders is None:
+            self._intruders = {}
+        fraction = float(fraction)
+        if fraction not in self._intruders:
+            seed = (self.seed * 0x9E3779B97F4A7C15 + INTRUDER_SEED_SALT) % (1 << 64)
+            self._intruders[fraction] = intruder_split(self.csr, fraction, seed)
+        return self._intruders[fraction]
 
     def mhat_device(self, ld=None) -> torch.Tensor:
         """float32 M-hat on the device (what Keras would see after its float32 cast)."""

@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from .._lib import call, ptr, stream_ptr
-from ..graph import rank_targets, topn_masked
+from ..graph import rank_cuts, rank_targets, topn_masked
 from ..sparse import CubeCSR
 from .model import CC_Recommender, SparseBatch
 
@@ -43,7 +43,7 @@ class MLRecommender:
     FUSED_MAX_N = 128        # cc_topn_masked_sigmoid_f32's limit (warp-per-cube streaming select)
 
     def _forward_chunks(self, csr: CubeCSR, *others: CubeCSR):
-        """The chunked forward of ``recommend_device`` and ``target_ranks_device``: yields ``(lo, hi, idx, ptr_, z,
+        """The chunked forward of ``recommend_device``, ``target_ranks_device`` and ``cut_ranks_device``: yields ``(lo, hi, idx, ptr_, z,
         rest)`` per chunk of ``self.chunk`` cubes, where ``idx`` / ``ptr_`` are rows [lo, hi) of ``csr`` on the device,
         ``z`` the (hi - lo, C) logits of ``decoder(encoder(rows))`` and ``rest`` one ``(idx, ptr)`` device pair of rows
         [lo, hi) per CSR in ``others``.  Chunk i+1's rows are uploaded on a copy stream while chunk i computes; nothing
@@ -120,15 +120,27 @@ class MLRecommender:
         would list it (for any ``amount``), or -1 if it is also visible.  Same chunked pipeline as ``recommend_device``
         with no host synchronisation; the ranks come from cc_rank_targets_f32 on the logits with the sigmoid fused
         in, so no probability row is written."""
-        if hidden.num_cubes != visible.num_cubes or hidden.num_cards != visible.num_cards:
-            raise ValueError("visible and hidden must hold the same cubes over the same cards")
-        if visible.num_cards != self.model.N:
-            raise ValueError(f"the cubes span {visible.num_cards} cards, the model {self.model.N}")
-        hp = np.ascontiguousarray(hidden.indptr, dtype=np.int64)
+        return self._ranks(visible, hidden, rank_targets, ("visible", "hidden"))
+
+    def cut_ranks_device(self, corrupted: CubeCSR, intruders: CubeCSR) -> torch.Tensor:
+        """Cut ranks, int32 aligned with ``intruders.indices``, on the device.  Cube b's ``corrupted`` cards (its own
+        plus its intruders) are the model input and the candidates; each of its ``intruders`` gets the 0-based slot at
+        which the cube's cut list -- its cards by ascending probability, ties to the smaller index, the order of
+        ``GraphRecommender.cuts`` and ``ml_recommend.py``'s lowest-scored lines -- would list it, or -1 if it is not one
+        of the corrupted cards.  Same chunked pipeline as ``recommend_device`` with no host synchronisation; the ranks
+        come from cc_rank_cuts_f32 on the logits with the sigmoid fused in."""
+        return self._ranks(corrupted, intruders, rank_cuts, ("corrupted", "intruders"))
+
+    def _ranks(self, inputs: CubeCSR, targets: CubeCSR, rank, names) -> torch.Tensor:
+        if targets.num_cubes != inputs.num_cubes or targets.num_cards != inputs.num_cards:
+            raise ValueError(f"{names[0]} and {names[1]} must hold the same cubes over the same cards")
+        if inputs.num_cards != self.model.N:
+            raise ValueError(f"the cubes span {inputs.num_cards} cards, the model {self.model.N}")
+        hp = np.ascontiguousarray(targets.indptr, dtype=np.int64)
         ranks = torch.empty(max(int(hp[-1]), 1), dtype=torch.int32, device=self.model.device)
-        for lo, hi, idx, ptr_, z, ((t_idx, t_ptr),) in self._forward_chunks(visible, hidden):
+        for lo, hi, idx, ptr_, z, ((t_idx, t_ptr),) in self._forward_chunks(inputs, targets):
             if hp[hi] > hp[lo]:
-                rank_targets(z, ptr_, idx, t_ptr, t_idx, sigmoid=True, out=ranks[int(hp[lo]):int(hp[hi])])
+                rank(z, ptr_, idx, t_ptr, t_idx, sigmoid=True, out=ranks[int(hp[lo]):int(hp[hi])])
         return ranks[:int(hp[-1])]
 
     def recommend(self, csr: CubeCSR, amount: int, copy: bool = True, want_cuts: bool = False):

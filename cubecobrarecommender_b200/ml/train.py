@@ -1,7 +1,8 @@
 """Drop-in for reference ``src/ml/train.py``.
 
     python -m cubecobrarecommender_b200.ml.train epochs batch_size name reg noise [seed] [--validation-split F]
-                                                 [--rank-at K1,K2,...] [--rank-baselines graph,popularity]
+                                                 [--rank-at K1,K2,...] [--rank-cuts]
+                                                 [--rank-baselines graph,popularity]
 
 Same positional arguments (reference train.py:28-38), same inputs (``data/maps/nameToId.json``,
 ``data/cube/*.json``, ``output/full_adj_mtx.npy``), same M-hat construction (train.py:69-71), loss and
@@ -94,25 +95,51 @@ def evaluate_recommendations(model, generator, *, at=(10, 50), holdout=0.2, grou
     the sums; the only host read is the final one.  Parameters, gradients, the tf32 shadow, Adam slots and step
     counters are left untouched, and no random stream is drawn from.  M-hat is built from every cube, the held-out
     ones included."""
+    return _ranking_eval("evaluate_recommendations", model, generator, at, group,
+                         lambda: generator.holdout_split(holdout), "target_ranks_device",
+                         lambda vis: generator.N_cards - np.diff(vis.indptr))
+
+
+def evaluate_cuts(model, generator, *, at=(10, 50), inject=0.2, group=None):
+    """Ranking quality of the cut list over every cube of ``generator``: each cube of s >= 1 cards gets
+    ``max(1, floor(inject * s + 0.5))`` intruders, cards of another cube that it does not hold
+    (``DataGenerator.intruder_split``: the same cards in every call), the model sees the corrupted cube, and every
+    intruder is placed where the cube's cut list (its cards by ascending probability, ties to the smaller index) would
+    list it, among the s + m cards of the corrupted cube.  A good cutter lists the intruders first.  ``model``: a
+    ``CC_Recommender`` (ranked through ``MLRecommender``) or any recommender with ``cut_ranks_device(corrupted,
+    intruders)`` -- ``MLRecommender``, ``graph.GraphRecommender`` (``simple_cuts``), ``graph.PopularityRecommender``.
+    Returns the keys of ``evaluate_recommendations`` (recall, NDCG and hit rate at each k in ``at``, ``"mrr"``,
+    ``"mpr"``: 0.5 for a random ordering), ``"cubes"`` (evaluated) and ``"skipped"`` (no cards, or no intruder
+    because the donor holds nothing the cube lacks).  Under ``torchrun`` each rank takes a contiguous shard of the
+    split made over the whole set and one all_reduce adds the sums; the only host read is the final one.  Parameters,
+    gradients, the tf32 shadow, Adam slots and step counters are left untouched, and no random stream is drawn from.
+    M-hat is built from every cube, the held-out ones included."""
+    return _ranking_eval("evaluate_cuts", model, generator, at, group, lambda: generator.intruder_split(inject),
+                         "cut_ranks_device", lambda corrupted: np.diff(corrupted.indptr))
+
+
+def _ranking_eval(what, model, generator, at, group, split, method, n_candidates):
+    """The metrics of ``ranking.ranking_sums`` over the ranks that recommender method ``method(inputs, targets)`` gives
+    this rank's shard of ``split() = (inputs, targets, evaluated)``; ``n_candidates(inputs)``: each cube's candidates."""
     import torch.distributed as dist
     from .inference import MLRecommender
     from .model import CC_Recommender
     from .ranking import metric_names, ranking_sums
     at = tuple(int(k) for k in at)
     if not at or min(at) < 1:
-        raise ValueError(f"evaluate_recommendations: every k in `at` must be >= 1, got {at}")
+        raise ValueError(f"{what}: every k in `at` must be >= 1, got {at}")
     world = dist.get_world_size(group) if dist.is_available() and dist.is_initialized() else 1
     rank = dist.get_rank(group) if world > 1 else 0
     k = generator.N_cubes
     if k < 1:
-        raise ValueError("evaluate_recommendations: the generator holds no cubes")
-    visible, hidden, _ = generator.holdout_split(holdout)
-    vis, hid = visible.shard(rank, world), hidden.shard(rank, world)          # the cubes of shard_range(k, rank, world)
+        raise ValueError(f"{what}: the generator holds no cubes")
+    inputs, targets, _ = split()
+    inp, tgt = inputs.shard(rank, world), targets.shard(rank, world)          # the cubes of shard_range(k, rank, world)
     rec = MLRecommender(model) if isinstance(model, CC_Recommender) else model
-    ranks = rec.target_ranks_device(vis, hid)
+    ranks = getattr(rec, method)(inp, tgt)
     dev = ranks.device
-    hp = torch.from_numpy(np.ascontiguousarray(hid.indptr, dtype=np.int64)).to(dev, non_blocking=True)
-    n_cand = torch.from_numpy(generator.N_cards - np.diff(vis.indptr)).to(dev, non_blocking=True)
+    hp = torch.from_numpy(np.ascontiguousarray(tgt.indptr, dtype=np.int64)).to(dev, non_blocking=True)
+    n_cand = torch.from_numpy(n_candidates(inp)).to(dev, non_blocking=True)
     sums = ranking_sums(ranks, hp, n_cand, at)
     if world > 1:
         dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
@@ -126,19 +153,24 @@ def evaluate_recommendations(model, generator, *, at=(10, 50), holdout=0.2, grou
 BASELINES = ("graph", "popularity")
 
 
-def ranking_baselines(train_generator, val_generator, *, names=BASELINES, at, holdout, group=None):
+def ranking_baselines(train_generator, val_generator, *, names=BASELINES, at, holdout=0.2, group=None, task="adds",
+                      inject=0.2):
     """``{name: evaluate_recommendations(...)}`` of simple recommenders on ``val_generator``'s cubes, the same hidden
     cards and metrics as the autoencoder's ranking evaluation, to read its numbers against.  ``"graph"``: the
     co-occurrence recommender (``simple_recs``, reference ``recommend.py:7-18``) with M built from the cubes of
     ``train_generator`` only, so no held-out co-occurrence leaks into it (the autoencoder's M-hat, by contrast, is built
     from every cube).  ``"popularity"``: the cards listed by the most training cubes, the same list for every cube.
-    Under ``torchrun`` every rank builds the whole graph (no all_reduce of the counts) and ranks its shard of the
-    validation cubes; the graph is freed before the function returns."""
+    ``task="cuts"``: ``{name: evaluate_cuts(..., inject=inject)}`` instead, the same intruders as the autoencoder's cut
+    evaluation; the graph cuts like ``simple_cuts`` (reference ``cut_cards.py:7-18``), popularity cuts the least-listed
+    cards first.  Under ``torchrun`` every rank builds the whole graph (no all_reduce of the counts) and ranks its shard
+    of the validation cubes; the graph is freed before the function returns."""
     from .. import graph as G
     names = tuple(names)
     unknown = [n for n in names if n not in BASELINES]
     if unknown:
         raise ValueError(f"unknown ranking baseline(s) {unknown}; choose from {list(BASELINES)}")
+    if task not in ("adds", "cuts"):
+        raise ValueError(f"task must be 'adds' or 'cuts', got {task!r}")
     out = {}
     for name in names:
         if name == "graph":
@@ -148,14 +180,18 @@ def ranking_baselines(train_generator, val_generator, *, names=BASELINES, at, ho
             del g                                           # the int32 counts go now, M with the recommender below
         else:
             rec = G.PopularityRecommender(train_generator.csr, train_generator.device)
-        out[name] = evaluate_recommendations(rec, val_generator, at=at, holdout=holdout, group=group)
+        if task == "adds":
+            out[name] = evaluate_recommendations(rec, val_generator, at=at, holdout=holdout, group=group)
+        else:
+            out[name] = evaluate_cuts(rec, val_generator, at=at, inject=inject, group=group)
         del rec
     return out
 
 
 def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch=None, max_cube_size=None,
         initial_epoch=0, checkpoint_dir=None, save_every=None, overflow_check_every=50, metrics=True,
-        validation_data=None, validation_split=0.0, validation_freq=1, ranking_at=None, ranking_holdout=0.2):
+        validation_data=None, validation_split=0.0, validation_freq=1, ranking_at=None, ranking_holdout=0.2,
+        ranking_cuts=False, ranking_inject=0.2):
     """``autoencoder.fit(generator, epochs=epochs)`` (reference train.py:99-102).  Returns the history
     ``[{"loss", "output_1_loss", "output_2_loss", "output_1_accuracy", "output_2_accuracy"}]`` per epoch (means over
     the epoch's steps, like Keras' progress line).  ``metrics`` mirrors ``compile(..., metrics=['accuracy'])`` (reference
@@ -173,9 +209,14 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
     progress line gain ``val_loss``, ``val_output_1_loss``, ``val_output_2_loss`` and, with ``metrics``, the two
     ``val_*_accuracy`` keys.  ``ranking_at`` (a sequence of k): the same epochs also run ``evaluate_recommendations``
     on the validation cubes with ``holdout=ranking_holdout`` and add ``val_recall_at_k``, ``val_ndcg_at_k`` and
-    ``val_hit_rate_at_k`` per k, ``val_mrr`` and ``val_mpr``."""
+    ``val_hit_rate_at_k`` per k, ``val_mrr`` and ``val_mpr``.  ``ranking_cuts`` (needs ``ranking_at``): the same
+    epochs also run ``evaluate_cuts`` with ``inject=ranking_inject`` and add ``val_cut_recall_at_k``,
+    ``val_cut_ndcg_at_k`` and ``val_cut_hit_rate_at_k`` per k, ``val_cut_mrr`` and ``val_cut_mpr``.  M-hat is built
+    from every cube, the validation cubes included."""
     import torch.distributed as dist
     from .engine import DAEEngine
+    if ranking_cuts and ranking_at is None:
+        raise ValueError("ranking_cuts reports the metrics of ranking_at: it needs ranking_at=(k1, k2, ...)")
     if ranking_at is not None:
         ranking_at = tuple(int(k) for k in ranking_at)
         if validation_data is None and not validation_split:
@@ -227,6 +268,9 @@ def fit(model, generator, epochs, reg, *, group=None, log=print, steps_per_epoch
             if ranking_at is not None:
                 rlogs = evaluate_recommendations(model, val, at=ranking_at, holdout=ranking_holdout, group=group)
                 history[-1].update({"val_" + key: v for key, v in rlogs.items() if key not in ("cubes", "skipped")})
+            if ranking_cuts:
+                clogs = evaluate_cuts(model, val, at=ranking_at, inject=ranking_inject, group=group)
+                history[-1].update({"val_cut_" + key: v for key, v in clogs.items() if key not in ("cubes", "skipped")})
         log(progress_line(nsteps, time.time() - t0, history[-1]))
         generator.on_epoch_end()
         if checkpoint_dir and save_every and (epoch + 1) % save_every == 0 and epoch + 1 < epochs:
@@ -243,6 +287,9 @@ def parse_args(argv):
     resume = "--resume" in args
     if resume:
         args.remove("--resume")
+    rank_cuts = "--rank-cuts" in args
+    if rank_cuts:
+        args.remove("--rank-cuts")
     flags = {"--save-every": None, "--validation-split": 0.0, "--rank-at": None, "--rank-baselines": None}
     for flag in flags:
         if flag in args:
@@ -253,7 +300,7 @@ def parse_args(argv):
             del args[i:i + 2]
     if len(args) < 5:
         raise SystemExit("usage: train.py epochs batch_size name reg noise [seed] [--save-every N] [--resume] "
-                         "[--validation-split F] [--rank-at K1,K2,...] [--rank-baselines graph,popularity]")
+                         "[--validation-split F] [--rank-at K1,K2,...] [--rank-cuts] [--rank-baselines graph,popularity]")
     split = float(flags["--validation-split"])
     if not 0.0 <= split < 1.0:
         raise SystemExit(f"--validation-split must lie in [0, 1), got {split}")
@@ -267,6 +314,8 @@ def parse_args(argv):
             raise SystemExit(f"--rank-at values must be >= 1, got {flags['--rank-at']}")
         if split == 0.0:
             raise SystemExit("--rank-at ranks the held-out cubes: it needs --validation-split F")
+    if rank_cuts and rank_at is None:
+        raise SystemExit("--rank-cuts reports the metrics of --rank-at: it needs --rank-at K1,K2,...")
     baselines = None
     if flags["--rank-baselines"] is not None:
         baselines = tuple(v for v in flags["--rank-baselines"].split(",") if v)
@@ -279,7 +328,7 @@ def parse_args(argv):
     return {"epochs": int(args[0]), "batch_size": int(args[1]), "name": args[2], "reg": float(args[3]),
             "noise": float(args[4]), "seed": int(args[5]) if len(args) == 6 else 0, "seed_given": len(args) == 6,
             "resume": resume, "save_every": int(flags["--save-every"]) if flags["--save-every"] is not None else None,
-            "validation_split": split, "rank_at": rank_at, "rank_baselines": baselines}
+            "validation_split": split, "rank_at": rank_at, "rank_cuts": rank_cuts, "rank_baselines": baselines}
 
 
 def main(argv=None):
@@ -289,8 +338,10 @@ def main(argv=None):
     ``--validation-split F`` holds the last fraction F of the cubes out of training and reports ``val_*`` losses and
     accuracies on them after every epoch, ``--rank-at 10,50`` adds the leave-k-out ranking metrics of those cubes
     (``val_recall_at_10``, ``val_ndcg_at_10``, ``val_hit_rate_at_10``, ..., ``val_mrr``, ``val_mpr``), and
-    ``--rank-baselines graph,popularity`` prints the same metrics of those baselines (``ranking_baselines``) on the
-    same cubes before the first epoch, one ``baseline <name> - recall_at_10: ...`` line each."""
+    ``--rank-cuts`` adds the same metrics of the cut list (``evaluate_cuts``: ``val_cut_recall_at_10``, ...,
+    ``val_cut_mpr``), and ``--rank-baselines graph,popularity`` prints the same metrics of those baselines
+    (``ranking_baselines``) on the same cubes before the first epoch, one ``baseline <name> - recall_at_10: ...`` line
+    each, followed with ``--rank-cuts`` by one ``baseline <name> cuts - recall_at_10: ...`` line each."""
     from ..non_ml import utils
     from .generator import DataGenerator
     from .model import CC_Recommender
@@ -332,9 +383,14 @@ def main(argv=None):
         for bname, logs in ranking_baselines(train_gen, val_gen, names=opts["rank_baselines"],
                                              at=opts["rank_at"], holdout=0.2).items():   # fit's ranking_holdout
             print(f"baseline {bname}" + "".join(f" - {key}: {logs[key]:.4f}" for key in metric_names(opts["rank_at"])))
+        if opts["rank_cuts"]:
+            for bname, logs in ranking_baselines(train_gen, val_gen, names=opts["rank_baselines"], at=opts["rank_at"],
+                                                 task="cuts", inject=0.2).items():          # fit's ranking_inject
+                print(f"baseline {bname} cuts" + "".join(f" - {key}: {logs[key]:.4f}"
+                                                         for key in metric_names(opts["rank_at"])))
         del train_gen, val_gen
     fit(autoencoder, generator, epochs, reg, initial_epoch=initial_epoch, checkpoint_dir=dest, save_every=save_every,
-        validation_split=opts["validation_split"], ranking_at=opts["rank_at"])
+        validation_split=opts["validation_split"], ranking_at=opts["rank_at"], ranking_cuts=opts["rank_cuts"])
     if not dist.is_initialized() or dist.get_rank() == 0:
         autoencoder.save(dest, epoch=epochs)
     if dist.is_initialized():

@@ -161,6 +161,24 @@ int cc_rank_targets_f32(const float* scores, int64_t ld, int32_t num_cards, int3
 int cc_rank_targets_f64(const double* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* mask_ptr,
                         const int32_t* mask_idx, const int64_t* target_ptr, const int32_t* target_idx,
                         int32_t* out_rank, void* stream);
+/* Cut ranks for offline evaluation of the cut list.  Per cube b the candidates are the distinct cards of [0, C) listed
+ * in row b of list (duplicate entries count once, out-of-range entries are ignored): exactly the set
+ * cc_topn_masked_*(mode_only_listed = 1) ranks.  For every entry p in [target_ptr[b], target_ptr[b+1]), out_rank[p]
+ * is the 0-based position of card target_idx[p] among them in the ascending order of
+ * cc_topn_masked_*(mode_only_listed = 1, descending = 0): smaller score first, ties -> smaller index first, with
+ * apply_sigmoid != 0 the float32 sigmoid of the logits (saturated probabilities tie).  So a target of rank r < n is
+ * the one that select returns at slot r.  A target not listed in row b, or outside [0, C), gets -1; duplicate target
+ * entries get the same rank.  Any number of listed cards and targets per row; C up to 100 000 and beyond (the list
+ * bitmap takes C / 8 bytes of shared memory).  NaN scores are outside the contract.  One CTA per cube, reading only
+ * the row's listed scores.  out_rank: int32 [target_ptr[batch]]. */
+int cc_rank_cuts_f32(const float* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* list_ptr,
+                     const int32_t* list_idx, const int64_t* target_ptr, const int32_t* target_idx, int apply_sigmoid,
+                     int32_t* out_rank, void* stream);
+/* The same ranks for float64 scores, in the order of cc_topn_masked_f64(mode_only_listed = 1, descending = 0).  No
+ * sigmoid.  ld == 0 means one score row shared by every cube (a popularity ranking); otherwise ld >= C. */
+int cc_rank_cuts_f64(const double* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* list_ptr,
+                     const int32_t* list_idx, const int64_t* target_ptr, const int32_t* target_idx, int32_t* out_rank,
+                     void* stream);
 /* Card similarity (src/scripts/similarity.py:25-29): out[r] = -cos(emb[r], emb[query]) with Keras' l2_normalize
  * (epsilon 1e-12), emb float32 [rows][ld >= dim]; rank ascending with cc_topn_masked_f32. */
 int cc_cosine_neg_f32(const float* emb, int64_t ld, int32_t rows, int32_t dim, int32_t query, float* out, void* stream);
