@@ -56,6 +56,7 @@ SIGNATURES = {
     "cc_rank_cuts_f32": (I, [P, I64, I32, I32, P, P, P, P, I, P, P]),
     "cc_rank_cuts_f64": (I, [P, I64, I32, I32, P, P, P, P, P, P]),
     "cc_cosine_neg_f32": (I, [P, I64, I32, I32, I32, P, P]),
+    "cc_cosine_neg_many_f32": (I, [P, I64, I32, P, I64, I32, I32, P, I64, P]),
     "cc_topn_masked_f64": (I, [P, I64, I32, I32, P, P, I, I, I32, P, I64, P, P, P, P]),
     # (3) noise
     "cc_alias_build_host": (I, [P, I32, P, P]),

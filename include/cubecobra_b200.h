@@ -182,6 +182,15 @@ int cc_rank_cuts_f64(const double* scores, int64_t ld, int32_t num_cards, int32_
 /* Card similarity (src/scripts/similarity.py:25-29): out[r] = -cos(emb[r], emb[query]) with Keras' l2_normalize
  * (epsilon 1e-12), emb float32 [rows][ld >= dim]; rank ascending with cc_topn_masked_f32. */
 int cc_cosine_neg_f32(const float* emb, int64_t ld, int32_t rows, int32_t dim, int32_t query, float* out, void* stream);
+/* Card / cube similarity for many queries at once: out[q * ldo + r] = -cos(queries[q], cands[r]) with Keras'
+ * l2_normalize (epsilon 1e-12), bit for bit the value cc_cosine_neg_f32 writes for that pair.  dim must be 64
+ * (the encoder's width).  num_queries == 0 is a no-op.  Rank each row ascending with cc_topn_masked_f32.
+ * queries float32 [num_queries][ldq], cands float32 [num_cands][ldc]: both 16-byte aligned with ldq and ldc multiples
+ * of 4 (the rows are read as float4).  out float32 [num_queries][ldo >= num_cands], any alignment (16-byte aligned
+ * rows, ldo % 4 == 0, are written as float4); columns [num_cands, ldo) are not written. */
+int cc_cosine_neg_many_f32(const float* queries, int64_t ldq, int32_t num_queries,
+                           const float* cands, int64_t ldc, int32_t num_cands, int32_t dim,
+                           float* out, int64_t ldo, void* stream);
 int cc_topn_masked_f64(const double* scores, int64_t ld, int32_t num_cards, int32_t batch, const int64_t* mask_ptr,
                        const int32_t* mask_idx, int mode_only_listed, int descending, int32_t n, void* workspace,
                        int64_t workspace_bytes, int32_t* out_ids, double* out_vals, int32_t* out_count, void* stream);
